@@ -22,6 +22,12 @@ N > 1   : weak scaling -- the frame grows to 1920 x (1080 N) and rank r renders 
 configs : at N = 1 the other BASELINE.json configs (#1 Cornell 256^2, #3 hall-principled, #5 instanced 4096^2) are measured
           in the same run and reported as sub-objects; `cpu_baseline` = the reference's AVX-512 renderer on the host cores
           this process may really use (affinity and cgroup quota), on a bounded sample of the same workload.
+--dump-outputs DIR : after the timed steps, the frame the timed path delivered after its last step is written as
+          DIR/raw.npy (linear radiance, (H, W, 4) float32) and, at N = 1, DIR/final.npy (the tonemapped plane).  Together
+          they stay within 64 * 10^6 bytes: an array that does not fit the rest of that budget is replaced by a fixed,
+          seeded sample of its pixels, (k, 4) (at 1080p: raw.npy whole, final.npy 93% of its pixels).  The scenes are
+          generated deterministically and the built-in sampler table is used, so the same arguments give the same inputs
+          on every run.
 """
 import argparse
 import json
@@ -55,7 +61,28 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-sample", default="auto", help="WxHxSPP of the bounded CPU sample (auto: by host core count)")
     ap.add_argument("--no-sort", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the planes of the last timed step to DIR/*.npy")
     return ap.parse_args()
+
+
+DUMP_BUDGET = 64 * 10 ** 6  # bytes, .npy headers included
+NPY_HEADER = 128
+
+
+def dump_outputs(out_dir, arrays):
+    """Save each (H, W, C) array as out_dir/<name>.npy in float32, in order; an array that does not fit what is left of
+    DUMP_BUDGET is saved as a fixed, seeded sample of its pixels instead."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    left = DUMP_BUDGET
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a, dtype=np.float32)
+        if a.nbytes + NPY_HEADER > left:
+            px = a.reshape(-1, a.shape[-1])
+            k = max(left - NPY_HEADER, 0) // px[0].nbytes
+            a = px[np.sort(np.random.default_rng(0).choice(len(px), k, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        left -= a.nbytes + NPY_HEADER
 
 
 def make_desc(workload, w, h):
@@ -377,7 +404,7 @@ def main():
     def gather():
         if use_dist:
             x, y, ww, hh = rect
-            rdist.gather_strips(frame_t[y:y + hh], w, H, dst=0)
+            return rdist.gather_strips(frame_t[y:y + hh], w, H, dst=0)
 
     it = 0
     for _ in range(max(a.warmup, 0)):
@@ -397,11 +424,12 @@ def main():
         e0.record()
     lib.rc_event_record(ctx, 0)
     done = 0
+    frame = None
     while done < a.steps:
         k = min(gather_every, a.steps - done)
         it = r.render(s, rect, it, k)  # k samples enqueued back to back, one sync
         done += k
-        gather()
+        frame = gather()
     lib.rc_event_record(ctx, 1)
     if use_dist:
         e1.record()
@@ -427,6 +455,11 @@ def main():
     else:
         rays_total, shadow_total, launches_total = float(rays_local), float(c["shadow_rays"]), launches_local
     value = rays_total / (ms * 1e-3) / 1e6
+    if a.dump_outputs and rank == 0:
+        if use_dist:
+            dump_outputs(a.dump_outputs, {"raw": frame.cpu().numpy()})
+        else:
+            dump_outputs(a.dump_outputs, {"raw": r.pixels(host.RAW), "final": r.pixels(host.FINAL)})
 
     # ---- e2e: one blocking public-API call per step + delivery of the frame to the host ----
     # The scene does not change between the samples of a progressive render, so it is uploaded once (timed separately

@@ -3,6 +3,8 @@
          with the reference's own committed sample output samples/00_basic.tga when /root/reference is present
   GPU  - the CUDA path reproduces them bit-for-bit from the arrays stored IN the fixture (no oracle library needed for
          the trace stages; the shading stages additionally need the reference's PMJ02 table, which only the oracle has)
+  GPU  - rc_render over the fixtures' arrays and the host layer's own path over small scenes render the planes stored in
+         tests/golden/cuda_images.npz bit-for-bit (built-in sampler table; no oracle library needed)
 """
 import ctypes as C
 import glob
@@ -11,13 +13,48 @@ import os
 import numpy as np
 import pytest
 
-from ray_b200 import capi, scenes
+from ray_b200 import capi, host, scenes
 from ray_b200.cuda import HIT_DTYPE, RAY_DTYPE, SHADOW_DTYPE
+from common import GOLDEN_ARRAYS as ARRAYS, STORED, maybe_oracle, render_golden, view_from_golden
 
-GOLDEN = sorted(glob.glob(os.path.join(os.path.dirname(__file__), "golden", "*.npz")))
 DESCS = {"cornell_48": lambda: scenes.cornell_box(48, 48), "zoo_64x48": lambda: scenes.material_zoo(64, 48)}
-ARRAYS = ["wnodes", "mtris", "tri_indices", "tri_materials", "materials", "mesh_instances", "vertices", "vtx_indices",
-          "lights", "li_indices", "light_cwnodes"]
+GOLDEN = sorted(p for p in glob.glob(os.path.join(os.path.dirname(__file__), "golden", "*.npz"))
+                if os.path.splitext(os.path.basename(p))[0] in DESCS)
+# Planes the CUDA path rendered when they were stored (tools/make_golden.py --cuda-images): the fixture scenes over the
+# reference-built arrays, and scenes built by the product's own host layer, both with the built-in sampler table.  Small
+# frames: float planes of Monte-Carlo noise barely compress.
+CUDA_IMAGES = os.path.join(os.path.dirname(__file__), "golden", "cuda_images.npz")
+GOLDEN_SPP = 4
+HOST_CASES = {
+    "host_cornell": (lambda: scenes.cornell_box(32, 32), 8),
+    "host_zoo": (lambda: scenes.material_zoo(32, 24), 4),
+    "host_textured": (lambda: scenes.textured(32, 24), 4),
+    "host_envmap_zoo": (lambda: scenes.envmap_zoo(32, 24), 4),
+    "host_hall_small": (lambda: scenes.hall("principled", 64, 36, floor_res=24, n_columns=4, col_seg=8, col_rings=6,
+                                            extra_lights=10), 4),
+    "host_instanced": (lambda: scenes.instanced(16, 400, 32, 32), 4),
+}
+
+
+def render_host_case(name):
+    """RendererBase::RenderScene over a scene built by the host layer; returns the planes a caller reads back (the
+    Cornell case also through the NLM denoiser, the zoo case also its AOVs) and the counters."""
+    make, spp = HOST_CASES[name]
+    desc = make()
+    w, h = desc.width, desc.height
+    r = host.Renderer(w, h)
+    s = scenes.build(desc, r.create_scene())
+    it = r.render(s, (0, 0, w, h), 0, spp)
+    out = {"raw": r.pixels(host.RAW), "final": r.pixels(host.FINAL)}
+    if name == "host_zoo":
+        out["base_color"], out["depth_normals"] = r.pixels(host.BASE_COLOR), r.pixels(host.DEPTH_NORMALS)
+    if name == "host_cornell":
+        r.denoise((0, 0, w, h), it)
+        out["nlm_raw"], out["nlm_final"] = r.pixels(host.RAW), r.pixels(host.FINAL)
+    counters = r.counters()
+    s.close()
+    r.close()
+    return out, counters, spp * w * h
 
 
 def _name(path):
@@ -88,24 +125,6 @@ def test_oracle_cornell_agrees_with_the_references_committed_sample_image(oracle
     sc.close()
 
 
-def _view_from_golden(g, keep):
-    v = capi.rc_scene_view()
-    for name in ARRAYS:
-        buf = np.ascontiguousarray(g["arr_" + name])
-        keep.append(buf)
-        stride = int(g["stride_" + name])
-        a = capi.rc_array(buf.ctypes.data if buf.size else None, buf.size // stride if stride else 0, stride)
-        setattr(v, name, a)
-    for name in ("tlas_root", "visible_lights_count", "blocker_lights_count", "env_map", "back_map", "env_light_index"):
-        setattr(v, name, int(g["s_" + name]))
-    v.sky_map_spread_angle = float(g["s_sky_map_spread_angle"])
-    for name in ("env_col", "back_col", "bounds_min", "bounds_max"):
-        arr = getattr(v, name)
-        for i, x in enumerate(g["s_" + name]):
-            arr[i] = float(x)
-    return v
-
-
 @pytest.mark.gpu
 @pytest.mark.parametrize("path", GOLDEN, ids=_name)
 def test_cuda_trace_reproduces_golden_without_the_oracle(path):
@@ -115,7 +134,7 @@ def test_cuda_trace_reproduces_golden_without_the_oracle(path):
     from ray_b200 import cuda
     g = np.load(path)
     keep = []
-    v = _view_from_golden(g, keep)
+    v = view_from_golden(g, keep)
     w, h = [int(x) for x in g["wh"]]
     ctx = cuda.Context(0)
     ctx.resize(w, h)
@@ -139,21 +158,32 @@ def test_cuda_trace_reproduces_golden_without_the_oracle(path):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("path", GOLDEN, ids=_name)
-def test_cuda_shading_and_image_reproduce_golden(path, oracle_mod):
+def test_cuda_shading_and_image_reproduce_golden(path):
+    """Primary shade, shadow rays and a 4-spp image from the fixture's arrays against the reference's outputs stored in
+    it; those need the reference's PMJ02 table, so without the oracle library the same stages run with the built-in
+    table and are checked against the digests stored in tests/golden/cuda_digests.json."""
     from ray_b200 import cuda
+    o = maybe_oracle()
     g = np.load(path)
     keep = []
-    v = _view_from_golden(g, keep)
+    v = view_from_golden(g, keep)
     w, h = [int(x) for x in g["wh"]]
     it = int(g["iteration"])
     ctx = cuda.Context(0)
     ctx.resize(w, h)
-    ctx.upload_tables(oracle_mod.pmj_table(), g["filter_table"])
+    ctx.upload_tables(o.pmj_table() if o else host.builtin_sampler_table(), g["filter_table"])
     ctx.upload_scene(v)
     cam = capi.rc_camera.from_buffer_copy(g["cam"].tobytes())
     p = ctx.make_pass(cam, (0, 0, w, h), it)
     ctx.fill_temp((0, 0, 0, 0))
     sec, sh = ctx.stage_shade(p, True, 0, g["primary_rays"].view(RAY_DTYPE), g["primary_hits_out"].view(HIT_DTYPE))
+    if o is None:
+        key = f"golden/{_name(path)}"
+        STORED.check(f"{key}/primary_shade", _by_xy(sec), _by_xy(sh), ctx.readback(capi.RC_BUF_TEMP))
+        ctx.stage_trace_shadow_rays(p, _by_xy(sh), cam.clamp_direct)
+        STORED.check(f"{key}/primary_shadow", ctx.readback(capi.RC_BUF_TEMP))
+        ctx.close()
+        return
     assert _by_xy(sec).tobytes() == _by_xy(g["secondary_rays"].view(RAY_DTYPE)).tobytes()
     assert _by_xy(sh).tobytes() == _by_xy(g["shadow_rays"].view(SHADOW_DTYPE)).tobytes()
     assert ctx.readback(capi.RC_BUF_TEMP).tobytes() == g["temp_after_primary_shade"].tobytes()
@@ -164,3 +194,33 @@ def test_cuda_shading_and_image_reproduce_golden(path, oracle_mod):
         ctx.render(ctx.make_pass(cam, (0, 0, w, h), i))
     assert ctx.readback(capi.RC_BUF_RAW).tobytes() == g["image_raw_4spp"].tobytes()
     ctx.close()
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("path", GOLDEN, ids=_name)
+def test_cuda_render_of_the_fixture_scene_is_unchanged(path):
+    """The whole wavefront (rc_render, ray sort on) over the fixture's reference-built arrays renders the stored planes,
+    bit for bit."""
+    g = np.load(path)
+    want = np.load(CUDA_IMAGES)
+    w, h = [int(x) for x in g["wh"]]
+    got, c = render_golden(g, GOLDEN_SPP)
+    assert c["primary_rays"] == GOLDEN_SPP * w * h
+    for plane, a in got.items():
+        assert np.isfinite(a).all()
+        ref = want[f"{_name(path)}_{plane}"]
+        assert a.tobytes() == ref.tobytes(), f"{plane}: L-inf {np.abs(a - ref).max()}"
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("name", list(HOST_CASES))
+def test_host_layer_render_is_unchanged(name):
+    """The product path (host layer: own SAH BVH8, light tree, camera, tables -> C-ABI -> kernels) renders the stored
+    planes, bit for bit."""
+    want = np.load(CUDA_IMAGES)
+    got, c, primary = render_host_case(name)
+    assert c["primary_rays"] == primary
+    for plane, a in got.items():
+        assert np.isfinite(a).all()
+        ref = want[f"{name}_{plane}"]
+        assert a.tobytes() == ref.tobytes(), f"{plane}: L-inf {np.abs(a - ref).max()}"

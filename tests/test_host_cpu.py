@@ -2,6 +2,7 @@
 WITHOUT a GPU by running the reference's own Ref:: traversal / shading code (oracle/_ref) over the arrays it builds,
 next to the reference's own Cpu::Scene built from the same description."""
 import ctypes as C
+import os
 
 import numpy as np
 import pytest
@@ -27,18 +28,24 @@ SCENES = {
 
 
 @pytest.fixture(scope="module", params=list(SCENES))
-def built(request, oracle_mod):
+def host_built(request):
     desc = SCENES[request.param]()
     hs = scenes.build(desc, host.Scene(None))
-    osc = scenes.build(desc, oracle_mod.Scene(wide=True))
     assert host.load_library().rh_error_count(None) == 0, host.load_library().rh_last_error(None)
-    yield request.param, desc, hs, osc
+    yield request.param, desc, hs
     hs.close()
+
+
+@pytest.fixture(scope="module")
+def built(host_built, oracle_mod):
+    name, desc, hs = host_built
+    osc = scenes.build(desc, oracle_mod.Scene(wide=True))
+    yield name, desc, hs, osc
     osc.close()
 
 
-def test_bvh8_structure(built):
-    name, desc, hs, osc = built
+def test_bvh8_structure(host_built):
+    name, desc, hs = host_built
     v = hs.view()
     nodes = _arr(v.wnodes, np.uint8).reshape(-1, 224)
     bmin = nodes[:, :96].copy().view(np.float32).reshape(-1, 3, 8)
@@ -91,21 +98,23 @@ def test_bvh8_structure(built):
     assert sorted(leaves) == list(range(v.mesh_instances.count))
 
 
+def _planes(mtris, tri_indices):
+    """triangle id -> its plane-form data, from the 8-wide triangle blocks and their triangle ids"""
+    m = mtris.reshape(-1, 3, 4, 8)  # block, {n,u,v}, comp, lane
+    ti = tri_indices.reshape(-1, 8)
+    out = {}
+    for b in range(len(ti)):
+        for lane in range(8):
+            out[int(ti[b, lane])] = m[b, :, :, lane].tobytes()
+    return out
+
+
 def test_triangle_planes_equal_the_references(built):
     """Same triangle => bit-identical plane-form data as Ray::PreprocessTri produced for the reference's own scene."""
     name, desc, hs, osc = built
     hv, ov = hs.view(), osc.view()
-
-    def planes(v):
-        m = _arr(v.mtris, np.float32).reshape(-1, 3, 4, 8)  # block, {n,u,v}, comp, lane
-        ti = _arr(v.tri_indices, np.uint32).reshape(-1, 8)
-        out = {}
-        for b in range(len(ti)):
-            for lane in range(8):
-                out[int(ti[b, lane])] = m[b, :, :, lane].tobytes()
-        return out
-
-    hp, op = planes(hv), planes(ov)
+    hp, op = _planes(_arr(hv.mtris, np.float32), _arr(hv.tri_indices, np.uint32)), \
+        _planes(_arr(ov.mtris, np.float32), _arr(ov.tri_indices, np.uint32))
     # global triangle ids are assigned identically (append order of meshes / index triples)
     common = set(hp) & set(op)
     assert len(common) >= desc.triangle_count() - 2
@@ -271,3 +280,45 @@ def test_view_render_reproduces_renderer_ref(oracle_mod):
     assert n_rays > 3 * 48 * 40 and n_shadow > 0
     ref.close()
     osc.close()
+
+
+GOLDEN = {"cornell_48": lambda: scenes.cornell_box(48, 48), "zoo_64x48": lambda: scenes.material_zoo(64, 48)}
+
+
+@pytest.mark.parametrize("name", list(GOLDEN))
+def test_host_layer_matches_the_references_stored_scene(name):
+    """The arrays the reference's own Cpu::Scene built for a small scene, stored in tests/golden/<name>.npz: the host
+    layer, fed the same description, gives the same triangle plane data, per-triangle materials, material records,
+    lights (type / flags word and colour), camera and pixel-filter table."""
+    g = np.load(os.path.join(os.path.dirname(__file__), "golden", name + ".npz"))
+    desc = GOLDEN[name]()
+    hs = scenes.build(desc, host.Scene(None))
+    assert host.load_library().rh_error_count(None) == 0, host.load_library().rh_last_error(None)
+    hv = hs.view()
+    hp = _planes(_arr(hv.mtris, np.float32), _arr(hv.tri_indices, np.uint32))
+    op = _planes(g["arr_mtris"].view(np.float32), g["arr_tri_indices"].view(np.uint32))
+    common = set(hp) & set(op)
+    assert len(common) >= desc.triangle_count() - 2
+    bad = [t for t in common if hp[t] != op[t]]
+    assert not bad, f"{len(bad)} triangles have different plane data"
+    assert _arr(hv.tri_materials, np.uint8).tobytes() == g["arr_tri_materials"].tobytes()
+    assert _arr(hv.materials, np.uint8).tobytes() == g["arr_materials"].tobytes()
+
+    hl = _arr(hv.lights, np.uint8).reshape(-1, 64)
+    ol = g["arr_lights"].reshape(-1, 64)
+    assert len(hl) == len(ol) and hv.li_indices.count * 4 == len(g["arr_li_indices"])
+    assert (hv.visible_lights_count, hv.blocker_lights_count) == \
+        (int(g["s_visible_lights_count"]), int(g["s_blocker_lights_count"]))
+    order_h, order_o = np.lexsort(hl[:, :16].T[::-1]), np.lexsort(ol[:, :16].T[::-1])
+    assert np.array_equal(hl[order_h][:, :16], ol[order_o][:, :16])
+
+    a, b = hs.camera(), capi.rc_camera.from_buffer_copy(g["cam"].tobytes())
+    for f, _ in capi.rc_camera._fields_:
+        x, y = getattr(a, f), getattr(b, f)
+        if hasattr(x, "__len__"):
+            assert np.allclose(list(x), list(y), rtol=0, atol=1e-7), f
+        else:
+            assert x == pytest.approx(y, rel=1e-6, abs=1e-7), f
+    if b.filter != capi.FILTER_BOX:
+        assert np.abs(host.builtin_filter_table(b.filter, desc.camera.filter_width) - g["filter_table"]).max() <= 2e-6
+    hs.close()

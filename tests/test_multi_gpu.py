@@ -8,6 +8,17 @@ from ray_b200 import capi, cuda, host, scenes
 
 pytestmark = pytest.mark.gpu
 
+# (input channels, output channels) of the 16 convolutions (rt_unet.cuh unet_layer; skip tensors included)
+UNET_SHAPES = [(9, 32), (32, 32), (32, 48), (48, 64), (64, 80), (80, 96), (96, 96), (160, 112), (112, 112), (160, 96),
+               (96, 96), (128, 64), (64, 64), (73, 64), (64, 32), (32, 3)]
+
+
+def _unet_layers(seed=5):
+    """A seeded weight set of the network's shapes: both sides run the same filter, whatever its weights."""
+    rng = np.random.default_rng(seed)
+    return [((rng.standard_normal((co, ci, 3, 3)) * np.sqrt(2.0 / (9 * ci))).astype(np.float16),
+             (rng.standard_normal(co) * 0.01).astype(np.float16)) for ci, co in UNET_SHAPES]
+
 
 def _n_devices():
     try:
@@ -20,7 +31,7 @@ def _n_devices():
 @pytest.mark.parametrize("make", [lambda: scenes.cornell_box(96, 70),
                                   lambda: scenes.hall("principled", 160, 90, floor_res=32, n_columns=6, col_seg=10,
                                                       col_rings=6, extra_lights=6)])
-def test_multi_device_frame_equals_single_device_frame(make, oracle_mod):
+def test_multi_device_frame_equals_single_device_frame(make):
     desc = make()
     w, h, spp = desc.width, desc.height, 5
     n = min(_n_devices(), 8)
@@ -55,7 +66,7 @@ def test_multi_device_frame_equals_single_device_frame(make, oracle_mod):
     many.denoise((0, 0, w, h), itsn[0])
     assert many.pixels(host.RAW).tobytes() == one.pixels(host.RAW).tobytes()
     # UNet denoise: the whole network runs on device 0 after its input planes were gathered there
-    layers = oracle_mod.unet_layers()
+    layers = _unet_layers()
     for r_, it_ in ((one, its1[0]), (many, itsn[0])):
         r_.set_unet_weights(layers, capi.RC_UNET_FP32)
         r_.denoise_unet((0, 0, w, h), it_)

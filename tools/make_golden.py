@@ -8,6 +8,10 @@ layouts rc_upload_scene takes, (b) inputs and the reference's outputs of the hot
   a 4-spp linear image of Ref's whole RenderScene   (needs the reference's PMJ02 table, so the GPU test that uses it is
                                                      skipped when the oracle library is absent)
 tests/test_golden.py checks the oracle against these (CPU, pins the oracle build) and the CUDA path against them (GPU).
+
+    python tools/make_golden.py --cuda-images OUT.npz   (on a B200; no oracle needed)
+stores what the CUDA path renders (tests/golden/cuda_images.npz): the fixture scenes over their stored arrays and the
+host-layer cases of tests/test_golden.py, so that every later change to the device or host code is checked against them.
 """
 import ctypes as C
 import os
@@ -80,6 +84,24 @@ def make(name, desc, iteration=2, spp=4):
     print(name, os.path.getsize(out) // 1024, "KiB", "rays", len(rays), "sec", len(sec), "shadow", len(sh))
 
 
+def cuda_images(out):
+    from common import render_golden
+    from test_golden import GOLDEN, GOLDEN_SPP, HOST_CASES, render_host_case
+    d = {}
+    for path in GOLDEN:
+        name = os.path.splitext(os.path.basename(path))[0]
+        planes, _ = render_golden(np.load(path), GOLDEN_SPP)
+        d.update({f"{name}_{k}": v for k, v in planes.items()})
+    for name in HOST_CASES:
+        planes, _, _ = render_host_case(name)
+        d.update({f"{name}_{k}": v for k, v in planes.items()})
+    np.savez_compressed(out, **d)
+    print(out, os.path.getsize(out) // 1024, "KiB", sorted(d))
+
+
 if __name__ == "__main__":
-    make("cornell_48", scenes.cornell_box(48, 48))
-    make("zoo_64x48", scenes.material_zoo(64, 48))
+    if len(sys.argv) == 3 and sys.argv[1] == "--cuda-images":
+        cuda_images(sys.argv[2])
+    else:
+        make("cornell_48", scenes.cornell_box(48, 48))
+        make("zoo_64x48", scenes.material_zoo(64, 48))
