@@ -96,7 +96,7 @@ typedef struct rc_scene_view {
 
 /* camera_t (reference Types.h:102-115) + pass_settings_t (Types.h:92-100), flattened to 32-bit fields. */
 typedef struct rc_camera {
-    uint32_t type;   /* eCamType: only Persp (0) is supported */
+    uint32_t type;   /* eCamType: Persp (0) or Geo (2, see rc_pass_desc); Ortho (1) is not supported */
     uint32_t filter; /* ePixelFilter */
     uint32_t view_transform; /* eViewTransform: Standard (0), or 1..9 (AgX / Filmic) after rc_set_view_lut */
     float fov, exposure, gamma, sensor_height;
@@ -116,18 +116,65 @@ typedef struct rc_rect {
     int32_t x, y, w, h;
 } rc_rect;
 
+/* Pass flags (rc_pass_desc::flags).  The reference-side binding maps ePassFlags onto the last five by name.
+ *
+ * Call the first surface a camera (or Geo) ray hits S.  The flags apply to every camera type; the rc_stage_* entry
+ * points ignore them.
+ *   RC_RENDER_SKIP_DIRECT     drops light reaching S in one segment: the bounce-0 shadow rays are not traced and the
+ *                             shading of bounce 1 adds no colour (emission, light hit, miss term).  Bounce-1 rays
+ *                             still continue.
+ *   RC_RENDER_SKIP_INDIRECT   keeps S's shadow-ray light and the bounce-1 colour, drops everything after: the bounce
+ *                             loop ends after the bounce-1 shading and the bounce-1 shadow rays are not traced.
+ *   RC_RENDER_LIGHTING_ONLY   at S the material's base colour (value x base texture) is white for shading; the
+ *                             base-colour AOV still records the real colour.
+ *   RC_RENDER_NO_BACKGROUND   camera rays that miss contribute (0,0,0) (their alpha is 0 already).
+ *   S's own emission (E0) is never dropped.  So, with the same seeds, per pixel and sample: full + E0_only ==
+ *   SKIP_INDIRECT + SKIP_DIRECT up to fp32 summation order, where E0_only sets both SKIP flags.
+ *   A light that casts no shadow adds its light at the surface it lights straight into that surface's colour, with no
+ *   shadow ray, so it cannot be told from emission there: rc_render refuses SKIP_DIRECT, SKIP_INDIRECT and OUTPUT_SH
+ *   (with rc_last_error) on a scene whose sampled lights include one with cast_shadow = 0.
+ *   RC_RENDER_OUTPUT_SH       also accumulates L1 spherical harmonics of the light arriving at S (RC_BUF_SH_*): per
+ *                             sample, the shadow-ray light of S (D) along the bounce-0 shadow-ray direction and
+ *                             everything that came back through the bounce-1 ray (I) along that ray's direction,
+ *                             sum of L * Y_k(w) with real SH in world space Y = {0.282095, 0.488603 w.y,
+ *                             0.488603 w.z, 0.488603 w.x}, times 2^exposure, kept as the same running mean as
+ *                             RC_BUF_FULL.  E0 is excluded, so where E0 = 0 coefficient 0 = 0.282095 * RAW rgb. */
 enum { RC_RENDER_ASYNC = 1 /* do not synchronise before returning; call rc_sync */,
-       RC_RENDER_NO_SORT = 2 /* skip the results-neutral inter-bounce ray sort */ };
+       RC_RENDER_NO_SORT = 2 /* skip the results-neutral inter-bounce ray sort */,
+       RC_RENDER_SKIP_DIRECT = 4, RC_RENDER_SKIP_INDIRECT = 8, RC_RENDER_LIGHTING_ONLY = 16,
+       RC_RENDER_NO_BACKGROUND = 32, RC_RENDER_OUTPUT_SH = 64 };
 
+/* Geo camera (cam.type == 2): lightmap baking of one mesh instance.  geo_instance names the instance, and
+ * [geo_tri_first, geo_tri_first + geo_tri_count) the global triangle range of its mesh; they are read only for a Geo
+ * camera and must lie inside the uploaded mesh_instances / tri_materials.  Ortho (1) is not supported.
+ *
+ * Texel (x, y) of the w x h frame covers texture coordinates [x, x+1) x [y, y+1) in texel units s = u*w, t = v*h,
+ * with NO v flip (the convention of the texture fetch, so a baked map binds as a texture of the same mesh as it is).
+ * For each active pixel of the rect the sample point is (x + jx, y + jy), (jx, jy) the pixel-filter draw of the
+ * perspective ray generator (the filter itself is ignored: box within the texel).  The winner is the LOWEST-indexed
+ * triangle of the range whose uv triangle contains the point: all three edge functions >= 0 after orienting by the sign
+ * of the uv area, in fp32 texel units, both windings, uvs not wrapped; triangles with |uv area| < 1e-12 texel^2 never
+ * win.  A winner emits one ray and its hit with no primary trace: P = xform * interpolated position, N = normalised
+ * world-space interpolated vertex normal, ray o = P, d = -N, c = 1, pdf = 1e6, camera depth, empty IOR stack,
+ * cone_width = world size of one texel on that triangle, cone_spread = 0; hit obj = geo_instance, prim = the global
+ * triangle id (front face), t = 0, u/v = weights of the triangle's 2nd/3rd vertex.  No winner: no ray, and the
+ * pixel's sample is 0.  So RAW alpha is the covered fraction of the samples (RGB premultiplied by it), uncovered texels
+ * stay 0, AOVs are written for covered samples only (normal N, depth 0), and the rays count as primary_rays.
+ * The per-texel candidate lists are built on the device at the first Geo pass and kept until the scene, the range or
+ * the frame size changes; a range whose texel-clamped uv boxes add up to more than 2^28 texel entries (1 GiB) is
+ * refused. */
 typedef struct rc_pass_desc {
     rc_camera cam;
     rc_rect rect;
     int32_t iteration; /* value of RegionContext::iteration AFTER the increment RenderScene does (>= 1) */
     uint32_t flags;
+    uint32_t geo_instance, geo_tri_first, geo_tri_count; /* Geo camera only */
 } rc_pass_desc;
 
+/* RC_BUF_SH_R/G/B: w x h RGBA32F planes holding the 4 L1 SH coefficients of one colour channel (RC_RENDER_OUTPUT_SH).
+ * They exist from the first pass with RC_RENDER_OUTPUT_SH on; rc_clear / rc_resize zero them. */
 enum { RC_BUF_FINAL = 0, RC_BUF_RAW = 1, RC_BUF_BASE_COLOR = 2, RC_BUF_DEPTH_NORMALS = 3, RC_BUF_FULL = 4,
-       RC_BUF_HALF = 5, RC_BUF_TEMP = 6 };
+       RC_BUF_HALF = 5, RC_BUF_TEMP = 6, RC_BUF_SH_R = 7, RC_BUF_SH_G = 8, RC_BUF_SH_B = 9 };
 
 /* Ray bookkeeping of the last rc_render calls since rc_reset_stats: what Mrays/s is computed from. */
 typedef struct rc_counters {
@@ -264,6 +311,9 @@ int rc_comm_get_counters(rc_comm *comm, rc_counters *out); /* summed over the de
 /* rays_out: ray_data_t[rect.w*rect.h] (72 B), hits_out: hit_data_t[...] (20 B); *count_out = rays generated. */
 int rc_stage_generate_primary_rays(rc_ctx *ctx, const rc_pass_desc *pass, void *rays_out, void *hits_out,
                                    int *count_out);
+/* the same for a Geo camera (pass->cam.type == 2): the rays and hit records of the covered texels; like a Geo pass of
+ * rc_render it also writes 0 into the RC_BUF_TEMP pixels of the uncovered texels */
+int rc_stage_generate_geo_rays(rc_ctx *ctx, const rc_pass_desc *pass, void *rays_out, void *hits_out, int *count_out);
 /* rays: in/out (transparency updates c/depth), hits: in/out.  trace_lights != 0 adds IntersectAreaLights. */
 int rc_stage_trace_rays(rc_ctx *ctx, const rc_pass_desc *pass, void *rays, void *hits, int count, int trace_lights);
 /* primary != 0: ShadePrimary (stores colour, updates AOVs) else ShadeSecondary (adds).  bounce selects the clamp as

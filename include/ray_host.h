@@ -72,6 +72,9 @@ void rh_render(rh_renderer *r, rh_scene *s, const rc_rect *rect, int *iteration,
 void rh_denoise(rh_renderer *r, const rc_rect *rect, int iteration);
 /* which: 0 get_pixels_ref, 1 get_raw_pixels_ref, 2 aux BaseColor, 3 aux DepthNormals; borrowed pointer */
 const float *rh_get_pixels(rh_renderer *r, int which, int *pitch);
+/* RendererBase::get_sh_data_ref: w*h shl1_data_t {coeff_r[4], coeff_g[4], coeff_b[4]} (row pitch *pitch = w) of the
+ * passes with camera_desc_t::output_sh; NULL when no such pass ran since the renderer was created or resized */
+const float *rh_get_sh_data(rh_renderer *r, int *pitch);
 void rh_get_stats(rh_renderer *r, uint64_t us[11]);
 void rh_reset_stats(rh_renderer *r);
 /* CUDA-backend extras */

@@ -195,7 +195,8 @@ class rc_rect(C.Structure):
 
 
 class rc_pass_desc(C.Structure):
-    _fields_ = [("cam", rc_camera), ("rect", rc_rect), ("iteration", i32), ("flags", u32)]
+    _fields_ = [("cam", rc_camera), ("rect", rc_rect), ("iteration", i32), ("flags", u32), ("geo_instance", u32),
+                ("geo_tri_first", u32), ("geo_tri_count", u32)]
 
 
 class rc_counters(C.Structure):
@@ -204,8 +205,12 @@ class rc_counters(C.Structure):
 
 
 RC_RENDER_ASYNC, RC_RENDER_NO_SORT = 1, 2
+RC_RENDER_SKIP_DIRECT, RC_RENDER_SKIP_INDIRECT, RC_RENDER_LIGHTING_ONLY, RC_RENDER_NO_BACKGROUND, RC_RENDER_OUTPUT_SH = \
+    4, 8, 16, 32, 64
+CAM_PERSP, CAM_ORTHO, CAM_GEO = 0, 1, 2
 RC_UNET_TENSOR_CORES, RC_UNET_FP32 = 0, 1
 RC_BUF_FINAL, RC_BUF_RAW, RC_BUF_BASE_COLOR, RC_BUF_DEPTH_NORMALS, RC_BUF_FULL, RC_BUF_HALF, RC_BUF_TEMP = range(7)
+RC_BUF_SH_R, RC_BUF_SH_G, RC_BUF_SH_B = 7, 8, 9
 
 
 def _apply(struct, kw):

@@ -162,7 +162,11 @@ void Renderer::FreeMirrors() {
     rc_host_free(raw_buf_);
     rc_host_free(base_color_buf_);
     rc_host_free(depth_normals_buf_);
+    rc_host_free(sh_buf_);
+    rc_host_free(sh_stage_);
     final_buf_ = raw_buf_ = base_color_buf_ = depth_normals_buf_ = nullptr;
+    sh_buf_ = nullptr;
+    sh_stage_ = nullptr;
 }
 
 void Renderer::Resize(const int w, const int h) {
@@ -192,7 +196,8 @@ void Renderer::Resize(const int w, const int h) {
     memset(raw_buf_, 0, n * sizeof(color_rgba_t));
     memset(base_color_buf_, 0, n * sizeof(color_rgba_t));
     memset(depth_normals_buf_, 0, n * sizeof(color_rgba_t));
-    final_dirty_ = raw_dirty_ = base_dirty_ = dn_dirty_ = true;
+    final_dirty_ = raw_dirty_ = base_dirty_ = dn_dirty_ = sh_dirty_ = true;
+    sh_used_ = false;
 }
 
 void Renderer::Clear(const color_rgba_t &c) {
@@ -201,6 +206,8 @@ void Renderer::Clear(const color_rgba_t &c) {
             log_->Error("Ray(CUDA): %s", rc_last_error(x));
         }
     }
+    frame_on_dev0_ = false;
+    final_dirty_ = raw_dirty_ = base_dirty_ = dn_dirty_ = sh_dirty_ = true;
 }
 
 SceneBase *Renderer::CreateScene() { return new Scene(log_, ctx_); }
@@ -262,14 +269,38 @@ void Renderer::RenderSceneBatch(const SceneBase &scene, RegionContext &region, c
         return;
     }
     const camera_t &cam = s.cams_[s.current_cam_._index];
+    rc_pass_desc p;
+    memset(&p, 0, sizeof(p));
+    if (cam.desc.type == RS_CAM_GEO) {
+        // the baked instance is resolved against the scene as it is now: it must still exist
+        const uint32_t mi = cam.desc.mi_index;
+        if (cam.desc.uv_index != 0) {
+            log_->Error("Ray(CUDA): Geo camera uv_index %u: meshes carry one uv set", cam.desc.uv_index);
+            return;
+        }
+        if (mi >= s.mesh_instances_.size() || !s.instance_alive_[mi] ||
+            s.mesh_instances_[mi].mesh_index >= s.meshes_.size() || !s.meshes_[s.mesh_instances_[mi].mesh_index].alive) {
+            log_->Error("Ray(CUDA): Geo camera: mesh instance %u does not exist", mi);
+            return;
+        }
+        const Scene::MeshRec &m = s.meshes_[s.mesh_instances_[mi].mesh_index];
+        p.geo_instance = mi;
+        p.geo_tri_first = m.tri_first;
+        p.geo_tri_count = m.tri_count;
+    }
     if (!Prepare(s, cam)) {
         return;
     }
-    rc_pass_desc p;
-    memset(&p, 0, sizeof(p));
     p.cam = cam.rc;
     p.rect = rc_rect{region.rect().x, region.rect().y, region.rect().w, region.rect().h};
     p.flags = render_flags_ | RC_RENDER_ASYNC;
+    p.flags |= (cam.desc.skip_direct_lighting ? RC_RENDER_SKIP_DIRECT : 0u) |
+               (cam.desc.skip_indirect_lighting ? RC_RENDER_SKIP_INDIRECT : 0u) |
+               (cam.desc.lighting_only ? RC_RENDER_LIGHTING_ONLY : 0u) |
+               (cam.desc.no_background ? RC_RENDER_NO_BACKGROUND : 0u) | (cam.desc.output_sh ? RC_RENDER_OUTPUT_SH : 0u);
+    if (cam.desc.output_sh) {
+        sh_used_ = true;
+    }
     for (int i = 0; i < count; ++i) {
         ++region.iteration;
         p.iteration = region.iteration;
@@ -291,7 +322,7 @@ void Renderer::RenderSceneBatch(const SceneBase &scene, RegionContext &region, c
         log_->Error("Ray(CUDA): %s", rc_last_error(ctx_));
     }
     frame_on_dev0_ = false;
-    final_dirty_ = raw_dirty_ = base_dirty_ = dn_dirty_ = true;
+    final_dirty_ = raw_dirty_ = base_dirty_ = dn_dirty_ = sh_dirty_ = true;
 }
 
 void Renderer::Readback(const int which, color_rgba_t *dst) const {
@@ -325,6 +356,39 @@ color_data_rgba_t Renderer::get_raw_pixels_ref() const {
     }
     return {raw_buf_, w_};
 }
+const shl1_data_t *Renderer::get_sh_data_ref() const {
+    if (!sh_used_ || w_ == 0 || h_ == 0) {
+        return nullptr;
+    }
+    if (sh_dirty_) {
+        const size_t n = size_t(w_) * h_;
+        if (!sh_buf_) {
+            sh_buf_ = static_cast<shl1_data_t *>(rc_host_alloc(n * sizeof(shl1_data_t)));
+            sh_stage_ = static_cast<color_rgba_t *>(rc_host_alloc(n * sizeof(color_rgba_t)));
+            if (!sh_buf_ || !sh_stage_) {
+                log_->Error("Ray(CUDA): failed to allocate the host SH mirror");
+                return nullptr;
+            }
+        }
+        for (int ch = 0; ch < 3; ++ch) {
+            // the SH planes stay where they were rendered (the denoisers do not gather them)
+            const rc_rect r{0, 0, w_, h_};
+            const int rc = comm_ ? rc_gather(comm_, RC_BUF_SH_R + ch, &r, &sh_stage_[0].v[0], w_)
+                                 : rc_readback(ctx_, RC_BUF_SH_R + ch, &r, &sh_stage_[0].v[0], w_);
+            if (rc != 0) {
+                log_->Error("Ray(CUDA): %s", comm_ ? rc_comm_last_error(comm_) : rc_last_error(ctx_));
+                return nullptr;
+            }
+            for (size_t i = 0; i < n; ++i) {
+                float *dst = ch == 0 ? sh_buf_[i].coeff_r : (ch == 1 ? sh_buf_[i].coeff_g : sh_buf_[i].coeff_b);
+                memcpy(dst, sh_stage_[i].v, 4 * sizeof(float));
+            }
+        }
+        sh_dirty_ = false;
+    }
+    return sh_buf_;
+}
+
 color_data_rgba_t Renderer::get_aux_pixels_ref(const eAUXBuffer buf) const {
     if (buf == eAUXBuffer::BaseColor) {
         if (base_dirty_) {

@@ -29,6 +29,11 @@ class Renderer final : public RendererBase {
     // host mirrors of the device planes, in pinned memory (rc_host_alloc) so a readback runs at full PCIe speed
     mutable color_rgba_t *final_buf_ = nullptr, *raw_buf_ = nullptr, *base_color_buf_ = nullptr, *depth_normals_buf_ = nullptr;
     mutable bool final_dirty_ = true, raw_dirty_ = true, base_dirty_ = true, dn_dirty_ = true;
+    // L1 SH of the bake passes (camera_desc_t::output_sh): w*h shl1_data_t, filled from the three RC_BUF_SH_* planes
+    mutable shl1_data_t *sh_buf_ = nullptr;
+    mutable color_rgba_t *sh_stage_ = nullptr; // one plane, staging for the interleave
+    mutable bool sh_dirty_ = true;
+    bool sh_used_ = false; // a pass with output_sh ran since the last Resize
 
     const Scene *uploaded_scene_ = nullptr;
     uint64_t uploaded_revision_ = 0;
@@ -57,7 +62,7 @@ class Renderer final : public RendererBase {
     color_data_rgba_t get_pixels_ref() const override;
     color_data_rgba_t get_raw_pixels_ref() const override;
     color_data_rgba_t get_aux_pixels_ref(eAUXBuffer buf) const override;
-    const shl1_data_t *get_sh_data_ref() const override { return nullptr; }
+    const shl1_data_t *get_sh_data_ref() const override;
     void Resize(int w, int h) override;
     void Clear(const color_rgba_t &c) override;
     SceneBase *CreateScene() override;

@@ -989,9 +989,13 @@ static void make_camera(const camera_desc_t &c, camera_t &cam, ILog *log) {
     cam.desc = c;
     rc_camera &r = cam.rc;
     memset(&r, 0, sizeof(r));
-    if (c.type != RS_CAM_PERSP) {
-        log->Error("Ray(CUDA): only perspective cameras are supported by the CUDA backend");
+    if (c.type != RS_CAM_PERSP && c.type != RS_CAM_GEO) {
+        log->Error("Ray(CUDA): only perspective and Geo cameras are supported by the CUDA backend");
     }
+    if (c.type == RS_CAM_GEO && c.uv_index != 0) {
+        log->Error("Ray(CUDA): Geo camera uv_index %u: meshes carry one uv set", c.uv_index);
+    }
+    // the pass-flag bools and mi_index stay in cam.desc: the renderer resolves them at render time
     // AgX / Filmic view transforms need their table (Cuda::Renderer::SetViewTransformLUT): checked at render time
     float o[3] = {c.origin[0], c.origin[1], c.origin[2]}, f[3] = {c.fwd[0], c.fwd[1], c.fwd[2]},
           u[3] = {c.up[0], c.up[1], c.up[2]};

@@ -151,6 +151,13 @@ const float *rh_get_pixels(rh_renderer *r, int which, int *pitch) {
     }
     return d.ptr ? d.ptr->v : nullptr;
 }
+const float *rh_get_sh_data(rh_renderer *r, int *pitch) {
+    const shl1_data_t *d = R(r)->get_sh_data_ref();
+    if (pitch) {
+        *pitch = d ? R(r)->size().first : 0;
+    }
+    return d ? d->coeff_r : nullptr;
+}
 void rh_get_stats(rh_renderer *r, uint64_t us[11]) {
     RendererBase::stats_t st = {};
     R(r)->GetStats(st);

@@ -16,8 +16,10 @@
 #include <vector>
 
 #include <cuda_runtime.h>
+#include <cub/device/device_scan.cuh>
 
 #include "rt_kernels.cuh"
+#include "rt_bake.cuh"
 #include "rt_trace.cuh"
 #include "rt_sort.cuh"
 #include "rt_denoise.cuh"
@@ -31,7 +33,9 @@ namespace {
 
 enum { EV_START = 0, EV_RAYGEN, EV_PTRACE, EV_PSHADE, EV_PSHADOW, EV_BOUNCE0 };
 constexpr int kEventsPerBounce = 4; // sort, trace, shade, shadow
-constexpr int kMaxEvents = EV_BOUNCE0 + kEventsPerBounce * kMaxBounces + 2;
+constexpr int EV_END = EV_BOUNCE0 + kEventsPerBounce * kMaxBounces;
+constexpr int EV_SH1 = EV_END + 2, EV_SH2 = EV_END + 3; // after k_sh_primary / k_sh_direct (RC_RENDER_OUTPUT_SH)
+constexpr int kMaxEvents = EV_END + 4;
 enum { KF_RAYGEN = 0, KF_TRACE, KF_SHADE, KF_SHADOW, KF_SORT, KF_RESOLVE, KF_COUNT };
 
 struct DevArray {
@@ -91,8 +95,19 @@ struct rc_ctx {
     bool have_scene = false;
     rc_scene_view scene_info{};
     uint32_t li_count = 0;
+    bool no_shadow_lights = false; // a light NEE samples casts no shadow (see rc_render)
     uint64_t scene_h2d_bytes = 0; // host->device bytes rc_upload_scene / rc_update_instances have copied so far
     std::map<uint32_t, uint32_t> tex_dense; // (storage << 28 | index) -> dense texture id of the uploaded scene
+
+    // Geo camera candidate lists (rt_bake.cuh) of one (scene upload, triangle range, frame size)
+    uint32_t *geo_offsets = nullptr, *geo_cursor = nullptr, *geo_list = nullptr;
+    size_t geo_list_cap = 0;
+    bool geo_valid = false;
+    uint32_t geo_first = 0, geo_count = 0;
+    // L1 SH planes (RC_BUF_SH_*) + per-sample scratch, allocated by the first RC_RENDER_OUTPUT_SH pass
+    ShPlanes sh{};
+    bool have_sh = false;
+    uint32_t sample_tag = 0;
 
     bool stats_enabled = true;
     std::vector<cudaEvent_t> events;
@@ -102,6 +117,7 @@ struct rc_ctx {
     };
     bool sample_pending = false;
     int pending_bounces = 0;
+    bool pending_sh = false;
     uint64_t stats_us[11] = {};
     double kernel_ms[KF_COUNT] = {};
     uint64_t kernel_launches[KF_COUNT] = {};
@@ -216,8 +232,22 @@ int fill_params(rc_ctx *ctx, const rc_pass_desc *pass, KParams &p) {
         return fail(ctx, "frame buffer has zero size (rc_resize)");
     }
     const rc_camera &c = pass->cam;
-    if (c.type != 0) {
-        return fail(ctx, "camera type %u is not supported by the CUDA backend (only Persp)", c.type);
+    if (c.type != 0 && c.type != 2) {
+        return fail(ctx, "camera type %u is not supported by the CUDA backend (Persp and Geo only)", c.type);
+    }
+    if (c.type == 2) {
+        if (pass->geo_instance >= ctx->mesh_instances.count) {
+            return fail(ctx, "Geo camera: mesh instance %u outside the %u uploaded", pass->geo_instance,
+                        ctx->mesh_instances.count);
+        }
+        const uint64_t end = uint64_t(pass->geo_tri_first) + pass->geo_tri_count;
+        if (end > ctx->tri_materials.count || 3 * end > ctx->vtx_indices.count) {
+            return fail(ctx, "Geo camera: triangle range [%u, %llu) outside the %u uploaded triangles", pass->geo_tri_first,
+                        (unsigned long long)end, ctx->tri_materials.count);
+        }
+        if (uint64_t(ctx->w) * ctx->h >= (1ull << 31)) {
+            return fail(ctx, "Geo camera: a %dx%d lightmap has more than 2^31 texels", ctx->w, ctx->h);
+        }
     }
     if (c.view_transform != 0 && (c.view_transform >= 16 || !ctx->d_view_lut[c.view_transform])) {
         return fail(ctx, "view transform %u needs its table (rc_set_view_lut)", c.view_transform);
@@ -448,13 +478,46 @@ const float4 *plane_of(const rc_ctx *ctx, int which) {
     case RC_BUF_FULL: return ctx->fb.full;
     case RC_BUF_HALF: return ctx->fb.half;
     case RC_BUF_TEMP: return ctx->fb.temp;
+    case RC_BUF_SH_R:
+    case RC_BUF_SH_G:
+    case RC_BUF_SH_B: return ctx->sh.coef[which - RC_BUF_SH_R];
     default: return nullptr;
     }
+}
+
+// plane `which` or an error naming why it is missing
+int plane_or_fail(rc_ctx *ctx, int which, const char *what, const float4 **out) {
+    *out = plane_of(ctx, which);
+    if (*out) {
+        return 0;
+    }
+    if (which >= RC_BUF_SH_R && which <= RC_BUF_SH_B) {
+        return fail(ctx, "%s: the SH planes exist from the first pass with RC_RENDER_OUTPUT_SH on", what);
+    }
+    return fail(ctx, "%s: unknown buffer %d", what, which);
 }
 
 float clamp_limit(float v) { return (v != 0.0f) ? 3.0f * v : 3.402823466e+38F; }
 
 int persistent_grid(const rc_ctx *ctx, int blocks_per_sm) { return ctx->num_sms * blocks_per_sm; }
+
+// Does next-event estimation sample a light that casts no shadow?  (lights reachable through li_indices; without
+// that list every light of the array is looked at)
+bool has_no_shadow_lights(const rc_scene_view *sv) {
+    const Light *l = static_cast<const Light *>(sv->lights.ptr);
+    if (!l || sv->lights.count == 0) {
+        return false;
+    }
+    const uint32_t *li = static_cast<const uint32_t *>(sv->li_indices.ptr);
+    const uint32_t n = li ? sv->li_indices.count : sv->lights.count;
+    for (uint32_t i = 0; i < n; ++i) {
+        const uint32_t k = li ? li[i] : i;
+        if (k < sv->lights.count && ((l[k].bits >> 4) & 1u) == 0) {
+            return true;
+        }
+    }
+    return false;
+}
 
 void record(rc_ctx *ctx, int ev) {
     if (ctx->stats_enabled) {
@@ -474,10 +537,11 @@ int harvest_stats(rc_ctx *ctx) {
         cudaEventElapsedTime(&v, ctx->events[a], ctx->events[b]);
         return double(v);
     };
-    const double raygen = ms(EV_START, EV_RAYGEN), ptrace = ms(EV_RAYGEN, EV_PTRACE), pshade = ms(EV_PTRACE, EV_PSHADE),
-                 pshadow = ms(EV_PSHADE, EV_PSHADOW);
+    const double raygen = ms(EV_START, EV_RAYGEN), ptrace = ms(EV_RAYGEN, EV_PTRACE), pshade = ms(EV_PTRACE, EV_PSHADE);
+    const double pshadow = ctx->pending_sh ? ms(EV_SH1, EV_PSHADOW) : ms(EV_PSHADE, EV_PSHADOW);
+    const double sh = ctx->pending_sh ? ms(EV_PSHADE, EV_SH1) + ms(EV_PSHADOW, EV_SH2) : 0.0;
     double ssort = 0, strace = 0, sshade = 0, sshadow = 0;
-    int prev = EV_PSHADOW;
+    int prev = ctx->pending_sh ? EV_SH2 : EV_PSHADOW;
     for (int b = 0; b < ctx->pending_bounces; ++b) {
         const int e = EV_BOUNCE0 + b * kEventsPerBounce;
         ssort += ms(prev, e + 0);
@@ -486,8 +550,7 @@ int harvest_stats(rc_ctx *ctx) {
         sshadow += ms(e + 2, e + 3);
         prev = e + 3;
     }
-    const int e_end = EV_BOUNCE0 + kEventsPerBounce * kMaxBounces;
-    const double resolve = ms(prev, e_end);
+    const double resolve = ms(prev, EV_END) + sh;
     ctx->stats_us[0] += uint64_t(raygen * 1000.0);
     ctx->stats_us[1] += uint64_t(ptrace * 1000.0);
     ctx->stats_us[2] += uint64_t(pshade * 1000.0);
@@ -518,11 +581,128 @@ void launch_shade(rc_ctx *ctx, int grid, cudaStream_t s, const KParams &p, RayBu
     }
 }
 
+GeoTarget geo_target(const rc_ctx *ctx, const rc_pass_desc *pass) {
+    return GeoTarget{static_cast<const Vertex *>(ctx->vertices.ptr), static_cast<const uint32_t *>(ctx->vtx_indices.ptr),
+                     pass->geo_tri_first, pass->geo_tri_count, ctx->w, ctx->h};
+}
+
+void free_geo_lists(rc_ctx *ctx) {
+    cudaFree(ctx->geo_offsets);
+    cudaFree(ctx->geo_cursor);
+    cudaFree(ctx->geo_list);
+    ctx->geo_offsets = ctx->geo_cursor = ctx->geo_list = nullptr;
+    ctx->geo_list_cap = 0;
+    ctx->geo_valid = false;
+}
+
+// Build (or reuse) the per-texel candidate lists of a Geo pass (rt_bake.cuh).  Blocking when it builds.
+int ensure_geo_lists(rc_ctx *ctx, const rc_pass_desc *pass) {
+    if (ctx->geo_valid && ctx->geo_first == pass->geo_tri_first && ctx->geo_count == pass->geo_tri_count) {
+        return 0;
+    }
+    ctx->geo_valid = false;
+    cudaStream_t s = ctx->stream;
+    const GeoTarget g = geo_target(ctx, pass);
+    const size_t n = size_t(ctx->w) * ctx->h;
+    if (!ctx->geo_offsets) {
+        if (dev_alloc(ctx, &ctx->geo_offsets, n + 1) || dev_alloc(ctx, &ctx->geo_cursor, n + 1)) {
+            return 1;
+        }
+    }
+    unsigned long long *d_total = nullptr, total = 0;
+    CU_CHECK(ctx, cudaMalloc(&d_total, sizeof(*d_total)));
+    cudaMemsetAsync(d_total, 0, sizeof(*d_total), s);
+    const uint32_t tris = g.tri_count;
+    if (tris != 0) {
+        k_geo_box_total<<<(tris + 255) / 256, 256, 0, s>>>(g, d_total);
+    }
+    const cudaError_t e = cudaMemcpyAsync(&total, d_total, sizeof(total), cudaMemcpyDeviceToHost, s);
+    cudaStreamSynchronize(s);
+    cudaFree(d_total);
+    CU_CHECK(ctx, e);
+    CU_CHECK(ctx, cudaGetLastError());
+    if (total > kGeoMaxEntries) {
+        return fail(ctx, "Geo camera: the candidate lists of triangles [%u, %u) at %dx%d would hold %llu entries, more than "
+                         "the 2^28 (1 GiB) the backend allows",
+                    g.tri_first, g.tri_first + g.tri_count, ctx->w, ctx->h, total);
+    }
+    if (total > ctx->geo_list_cap || !ctx->geo_list) {
+        if (dev_alloc(ctx, &ctx->geo_list, size_t(total ? total : 1))) {
+            return 1;
+        }
+        ctx->geo_list_cap = size_t(total);
+    }
+    CU_CHECK(ctx, cudaMemsetAsync(ctx->geo_cursor, 0, (n + 1) * sizeof(uint32_t), s));
+    const int warp_blocks = int(std::min<uint64_t>((uint64_t(tris) * 32 + 255) / 256, uint64_t(ctx->num_sms) * 64));
+    if (tris != 0) {
+        k_geo_walk<false><<<warp_blocks, 256, 0, s>>>(g, ctx->geo_cursor, nullptr);
+    }
+    size_t temp_bytes = 0;
+    cub::DeviceScan::ExclusiveSum(nullptr, temp_bytes, ctx->geo_cursor, ctx->geo_offsets, int(n + 1), s);
+    void *d_temp = nullptr;
+    CU_CHECK(ctx, cudaMalloc(&d_temp, temp_bytes ? temp_bytes : 16));
+    cub::DeviceScan::ExclusiveSum(d_temp, temp_bytes, ctx->geo_cursor, ctx->geo_offsets, int(n + 1), s);
+    const cudaError_t e2 = cudaMemcpyAsync(ctx->geo_cursor, ctx->geo_offsets, n * sizeof(uint32_t), cudaMemcpyDeviceToDevice, s);
+    if (e2 == cudaSuccess && tris != 0) {
+        k_geo_walk<true><<<warp_blocks, 256, 0, s>>>(g, ctx->geo_cursor, ctx->geo_list);
+    }
+    cudaStreamSynchronize(s);
+    cudaFree(d_temp);
+    CU_CHECK(ctx, e2);
+    CU_CHECK(ctx, cudaGetLastError());
+    ctx->geo_first = pass->geo_tri_first;
+    ctx->geo_count = pass->geo_tri_count;
+    ctx->geo_valid = true;
+    return 0;
+}
+
+GeoParams geo_params(const rc_ctx *ctx, const rc_pass_desc *pass) {
+    return GeoParams{geo_target(ctx, pass), ctx->geo_offsets, ctx->geo_list,
+                     static_cast<const MeshInstance *>(ctx->mesh_instances.ptr) + pass->geo_instance, pass->geo_instance};
+}
+
+void free_sh(rc_ctx *ctx) {
+    for (float4 *b : {ctx->sh.coef[0], ctx->sh.coef[1], ctx->sh.coef[2], ctx->sh.e0, ctx->sh.direct, ctx->sh.dir0, ctx->sh.dir1}) {
+        cudaFree(b);
+    }
+    ctx->sh = ShPlanes{};
+    ctx->have_sh = false;
+}
+
+// the SH planes (zeroed) + scratch at the current frame size
+int alloc_sh(rc_ctx *ctx) {
+    const size_t n = size_t(ctx->w) * ctx->h;
+    free_sh(ctx);
+    for (float4 **b : {&ctx->sh.coef[0], &ctx->sh.coef[1], &ctx->sh.coef[2], &ctx->sh.e0, &ctx->sh.direct, &ctx->sh.dir0,
+                       &ctx->sh.dir1}) {
+        if (dev_alloc(ctx, b, n)) {
+            free_sh(ctx);
+            return 1;
+        }
+        CU_CHECK(ctx, cudaMemsetAsync(*b, 0, n * sizeof(float4), ctx->stream));
+    }
+    ctx->have_sh = true;
+    return 0;
+}
+
 // Enqueue the kernels of one sample.
 int enqueue_sample(rc_ctx *ctx, const rc_pass_desc *pass, KParams &p) {
     cudaStream_t s = ctx->stream;
     const int max_bounces = p.ps.max_total_depth;
     const bool do_sort = (pass->flags & RC_RENDER_NO_SORT) == 0;
+    const bool geo = pass->cam.type == 2;
+    const bool skip_direct = (pass->flags & RC_RENDER_SKIP_DIRECT) != 0;
+    // RC_RENDER_SKIP_INDIRECT: the bounce loop ends after the bounce-1 shading
+    const int last_bounce = (pass->flags & RC_RENDER_SKIP_INDIRECT) ? std::min(1, max_bounces) : max_bounces;
+    const bool want_sh = (pass->flags & RC_RENDER_OUTPUT_SH) != 0;
+    uint32_t shadow_traced = ~0u;
+    if (skip_direct) {
+        shadow_traced &= ~1u;
+    }
+    if (pass->flags & RC_RENDER_SKIP_INDIRECT) {
+        shadow_traced &= 1u;
+    }
+    const uint32_t tag = ++ctx->sample_tag;
 
     if (ctx->sample_pending && ctx->stats_enabled) {
         // event slots are reused per sample: collect the previous sample's timings first.  Without statistics nothing
@@ -544,7 +724,11 @@ int enqueue_sample(rc_ctx *ctx, const rc_pass_desc *pass, KParams &p) {
 
     const int n_pix_tiles = ((p.rect_w + 7) / 8) * ((p.rect_h + 3) / 4);
     const int raygen_blocks = (n_pix_tiles * 32 + 255) / 256;
-    k_raygen<<<raygen_blocks, 256, 0, s>>>(p, ctx->rays[0], ctx->hits);
+    if (geo) {
+        k_raygen_geo<<<raygen_blocks, 256, 0, s>>>(p, geo_params(ctx, pass), ctx->rays[0], ctx->hits);
+    } else {
+        k_raygen<<<raygen_blocks, 256, 0, s>>>(p, ctx->rays[0], ctx->hits);
+    }
     ctx->kernel_launches[KF_RAYGEN]++;
     record(ctx, EV_RAYGEN);
 
@@ -552,7 +736,7 @@ int enqueue_sample(rc_ctx *ctx, const rc_pass_desc *pass, KParams &p) {
     const int shade_grid = persistent_grid(ctx, RT_SHADE_BLOCKS);
     const bool have_geo = ctx->scene_info.tlas_root != 0xffffffffu;
 
-    if (have_geo) {
+    if (have_geo && !geo) { // k_raygen_geo writes the hit records itself
         k_trace_closest<false, false><<<trace_grid, kTraceThreads, 0, s>>>(p, ctx->rays[0], ctx->hits, 0, ctx->trace_fin_min);
         ctx->kernel_launches[KF_TRACE]++;
     }
@@ -561,19 +745,37 @@ int enqueue_sample(rc_ctx *ctx, const rc_pass_desc *pass, KParams &p) {
     const float mix_factor = 1.0f / float(p.iteration);
     {
         const float lim = clamp_limit(p.ps.clamp_direct);
-        launch_shade<true>(ctx, shade_grid, s, p, ctx->rays[0], ctx->rays[1], 0, lim, lim, mix_factor);
+        KParams pp = p;
+        pp.flags = (pass->flags & RC_RENDER_LIGHTING_ONLY) ? KP_LIGHTING_ONLY : 0u;
+        launch_shade<true>(ctx, shade_grid, s, pp, ctx->rays[0], ctx->rays[1], 0, lim, lim, mix_factor);
         ctx->kernel_launches[KF_SHADE]++;
+        if (pass->flags & RC_RENDER_NO_BACKGROUND) {
+            k_no_background<<<shade_grid, 256, 0, s>>>(p, ctx->rays[0], ctx->hits);
+            ctx->kernel_launches[KF_SHADE]++;
+        }
     }
     record(ctx, EV_PSHADE);
+    const int n_rect = p.rect_w * p.rect_h;
+    const int sh_grid = std::min((n_rect + 255) / 256, ctx->num_sms * 8);
+    if (want_sh) { // before the sort of bounce 1 reorders list 1
+        k_sh_primary<<<sh_grid, 256, 0, s>>>(p, ctx->sh, ctx->rays[1], tag);
+        ctx->kernel_launches[KF_RESOLVE]++;
+        record(ctx, EV_SH1);
+    }
 
-    if (have_geo) {
+    if (have_geo && !skip_direct) {
         k_trace_shadow<<<trace_grid, kTraceThreads, 0, s>>>(p, ctx->shadow, 0, clamp_limit(p.ps.clamp_direct), ctx->trace_fin_min);
         ctx->kernel_launches[KF_SHADOW]++;
     }
     record(ctx, EV_PSHADOW);
+    if (want_sh) {
+        k_sh_direct<<<sh_grid, 256, 0, s>>>(p, ctx->sh, ctx->shadow, tag);
+        ctx->kernel_launches[KF_RESOLVE]++;
+        record(ctx, EV_SH2);
+    }
 
     int cur = 1; // list index holding the rays of the current bounce
-    for (int bounce = 1; bounce <= max_bounces; ++bounce) {
+    for (int bounce = 1; bounce <= last_bounce; ++bounce) {
         const int e = EV_BOUNCE0 + (bounce - 1) * kEventsPerBounce;
         if (do_sort) {
             sort_rays(ctx->sort, p, ctx->rays[cur], ctx->rays[cur ^ 1], bounce, ctx->num_sms, /*have_hist*/ true,
@@ -595,12 +797,14 @@ int enqueue_sample(rc_ctx *ctx, const rc_pass_desc *pass, KParams &p) {
         record(ctx, e + 1);
         {
             const float cd = (bounce == 1) ? p.ps.clamp_direct : p.ps.clamp_indirect;
-            launch_shade<false>(ctx, shade_grid, s, p, ctx->rays[cur], ctx->rays[cur ^ 1], bounce, clamp_limit(cd),
+            KParams pp = p;
+            pp.flags = (bounce == 1 && skip_direct) ? KP_DROP_COL : 0u;
+            launch_shade<false>(ctx, shade_grid, s, pp, ctx->rays[cur], ctx->rays[cur ^ 1], bounce, clamp_limit(cd),
                                 clamp_limit(p.ps.clamp_indirect), mix_factor);
             ctx->kernel_launches[KF_SHADE]++;
         }
         record(ctx, e + 2);
-        if (have_geo) {
+        if (have_geo && ((shadow_traced >> bounce) & 1u)) {
             k_trace_shadow<<<trace_grid, kTraceThreads, 0, s>>>(p, ctx->shadow, bounce, clamp_limit(p.ps.clamp_indirect), ctx->trace_fin_min);
             ctx->kernel_launches[KF_SHADOW]++;
         }
@@ -616,17 +820,21 @@ int enqueue_sample(rc_ctx *ctx, const rc_pass_desc *pass, KParams &p) {
         const float vt = p.iteration > pass->cam.min_samples
                              ? 0.5f * pass->cam.variance_threshold * pass->cam.variance_threshold
                              : 0.0f;
-        const int n = p.rect_w * p.rect_h;
         const DisplayXf xf{pass->cam.view_transform ? ctx->d_view_lut[pass->cam.view_transform] : nullptr, inv_gamma};
-        k_resolve<<<(n + 255) / 256, 256, 0, s>>>(p, exposure_mul, mix_factor, half_mix_factor, is_class_a, xf, vt);
+        if (want_sh) { // reads temp before k_resolve overwrites it with the variance
+            k_sh_resolve<<<(n_rect + 255) / 256, 256, 0, s>>>(p, ctx->sh, tag, exposure_mul, mix_factor);
+            ctx->kernel_launches[KF_RESOLVE]++;
+        }
+        k_resolve<<<(n_rect + 255) / 256, 256, 0, s>>>(p, exposure_mul, mix_factor, half_mix_factor, is_class_a, xf, vt);
         ctx->last_xf = xf;
         ctx->last_variance_threshold = vt;
         ctx->kernel_launches[KF_RESOLVE]++;
-        k_accumulate_totals<<<1, 32, 0, s>>>(p, max_bounces);
+        k_accumulate_totals<<<1, 32, 0, s>>>(p, last_bounce, shadow_traced);
     }
-    record(ctx, EV_BOUNCE0 + kEventsPerBounce * kMaxBounces);
+    record(ctx, EV_END);
     ctx->sample_pending = ctx->stats_enabled;
-    ctx->pending_bounces = max_bounces;
+    ctx->pending_bounces = last_bounce;
+    ctx->pending_sh = want_sh;
     CU_CHECK(ctx, cudaGetLastError());
     return 0;
 }
@@ -865,6 +1073,8 @@ void rc_destroy(rc_ctx *ctx) {
     cudaFree(ctx->d_filter_table);
     cudaFree(ctx->d_srgb_lut);
     cudaFree(ctx->nlm_scratch);
+    free_geo_lists(ctx);
+    free_sh(ctx);
     for (int i = 0; i < kUNetLayers; ++i) {
         cudaFree(ctx->unet_w[i]);
         cudaFree(ctx->unet_b[i]);
@@ -909,6 +1119,9 @@ int rc_resize(rc_ctx *ctx, int w, int h) {
     // for a zero-size frame), not pointing at freed or mis-sized planes
     ctx->w = ctx->h = ctx->fb.w = ctx->fb.h = 0;
     ctx->ray_capacity = 0;
+    free_geo_lists(ctx);
+    const bool had_sh = ctx->have_sh;
+    free_sh(ctx);
     if (dev_alloc(ctx, &ctx->fb.temp, n) || dev_alloc(ctx, &ctx->fb.full, n) || dev_alloc(ctx, &ctx->fb.half, n) ||
         dev_alloc(ctx, &ctx->fb.raw, n) || dev_alloc(ctx, &ctx->fb.final, n) || dev_alloc(ctx, &ctx->fb.base_color, n) ||
         dev_alloc(ctx, &ctx->fb.depth_normals, n) || dev_alloc(ctx, &ctx->fb.required_samples, n)) {
@@ -934,6 +1147,9 @@ int rc_resize(rc_ctx *ctx, int w, int h) {
     ctx->fb.h = h;
     ctx->w = w;
     ctx->h = h;
+    if (had_sh && n && alloc_sh(ctx)) {
+        return 1;
+    }
     CU_CHECK(ctx, cudaStreamSynchronize(ctx->stream));
     return 0;
 }
@@ -956,6 +1172,11 @@ int rc_clear(rc_ctx *ctx, const float rgba[4]) {
     const float4 v = make_float4(rgba[0], rgba[1], rgba[2], rgba[3]);
     k_fill4<<<ctx->num_sms * 4, 256, 0, ctx->stream>>>(ctx->fb.full, v, n);
     k_fill4<<<ctx->num_sms * 4, 256, 0, ctx->stream>>>(ctx->fb.half, v, n);
+    if (ctx->have_sh) {
+        for (float4 *c : ctx->sh.coef) {
+            CU_CHECK(ctx, cudaMemsetAsync(c, 0, n * sizeof(float4), ctx->stream));
+        }
+    }
     CU_CHECK(ctx, cudaMemsetAsync(ctx->fb.required_samples, 0xff, n * sizeof(uint16_t), ctx->stream));
     CU_CHECK(ctx, cudaStreamSynchronize(ctx->stream));
     return 0;
@@ -1181,7 +1402,9 @@ int rc_upload_scene(rc_ctx *ctx, const rc_scene_view *sv) {
         q = nullptr;
     }
     ctx->li_count = sv->li_indices.count;
+    ctx->no_shadow_lights = has_no_shadow_lights(sv);
     ctx->tex_dense = dense;
+    ctx->geo_valid = false; // the candidate lists depend on the uvs of the uploaded triangles
     set_sort_bounds(ctx->sort, sv->bounds_min, sv->bounds_max);
     if (build_traversal_copies(ctx, sv)) {
         return 1;
@@ -1355,6 +1578,7 @@ int rc_update_instances(rc_ctx *ctx, const rc_scene_view *sv, uint32_t first_nod
     memcpy(info.bounds_min, sv->bounds_min, sizeof(info.bounds_min));
     memcpy(info.bounds_max, sv->bounds_max, sizeof(info.bounds_max));
     ctx->li_count = sv->li_indices.count;
+    ctx->no_shadow_lights = has_no_shadow_lights(sv);
     set_sort_bounds(ctx->sort, sv->bounds_min, sv->bounds_max);
     ctx->have_scene = true;
     return 0;
@@ -1367,6 +1591,19 @@ int rc_render(rc_ctx *ctx, const rc_pass_desc *pass) {
     cudaSetDevice(ctx->device);
     KParams p;
     if (fill_params(ctx, pass, p)) {
+        return 1;
+    }
+    const uint32_t split_flags = RC_RENDER_SKIP_DIRECT | RC_RENDER_SKIP_INDIRECT | RC_RENDER_OUTPUT_SH;
+    if ((pass->flags & split_flags) && ctx->no_shadow_lights) {
+        // the shading adds such a light's contribution straight into the colour of the surface it lights, with no
+        // shadow ray: the kernels cannot tell it from that surface's emission, so the split would be wrong
+        return fail(ctx, "RC_RENDER_SKIP_DIRECT / SKIP_INDIRECT / OUTPUT_SH need every sampled light to cast shadows; "
+                         "the scene has a light with cast_shadow = 0");
+    }
+    if (pass->cam.type == 2 && ensure_geo_lists(ctx, pass)) {
+        return 1;
+    }
+    if ((pass->flags & RC_RENDER_OUTPUT_SH) && !ctx->have_sh && alloc_sh(ctx)) {
         return 1;
     }
     if (enqueue_sample(ctx, pass, p)) {
@@ -1893,15 +2130,8 @@ int rc_readback(rc_ctx *ctx, int which, const rc_rect *rect, float *dst, int pit
     }
     cudaSetDevice(ctx->device);
     const float4 *src = nullptr;
-    switch (which) {
-    case RC_BUF_FINAL: src = ctx->fb.final; break;
-    case RC_BUF_RAW: src = ctx->fb.raw; break;
-    case RC_BUF_BASE_COLOR: src = ctx->fb.base_color; break;
-    case RC_BUF_DEPTH_NORMALS: src = ctx->fb.depth_normals; break;
-    case RC_BUF_FULL: src = ctx->fb.full; break;
-    case RC_BUF_HALF: src = ctx->fb.half; break;
-    case RC_BUF_TEMP: src = ctx->fb.temp; break;
-    default: return fail(ctx, "rc_readback: unknown buffer %d", which);
+    if (plane_or_fail(ctx, which, "rc_readback", &src)) {
+        return 1;
     }
     if (rect->x < 0 || rect->y < 0 || rect->w <= 0 || rect->h <= 0 || rect->x + rect->w > ctx->w ||
         rect->y + rect->h > ctx->h || pitch < rect->w) {
@@ -1919,9 +2149,9 @@ int rc_readback_async(rc_ctx *ctx, int which, const rc_rect *rect, float *dst, i
         return fail(ctx, "rc_readback_async: null argument");
     }
     cudaSetDevice(ctx->device);
-    const float4 *src = plane_of(ctx, which);
-    if (!src) {
-        return fail(ctx, "rc_readback_async: unknown buffer %d", which);
+    const float4 *src = nullptr;
+    if (plane_or_fail(ctx, which, "rc_readback_async", &src)) {
+        return 1;
     }
     if (rect->x < 0 || rect->y < 0 || rect->w <= 0 || rect->h <= 0 || rect->x + rect->w > ctx->w ||
         rect->y + rect->h > ctx->h || pitch < rect->w) {
@@ -2078,6 +2308,13 @@ int rc_comm_render(rc_comm *comm, const rc_pass_desc *pass) {
                              comm->ctxs[0]->w, comm->ctxs[0]->h);
         }
         rc_pass_desc p = *pass;
+        if ((pass->flags & RC_RENDER_OUTPUT_SH) && !ctx->have_sh) {
+            // every device holds the planes, also one whose band this pass does not touch: rc_gather reads them all
+            cudaSetDevice(ctx->device);
+            if (alloc_sh(ctx) || cudaStreamSynchronize(ctx->stream) != cudaSuccess) {
+                return comm_fail(comm, "device %d: %s", ctx->device, rc_last_error(ctx));
+            }
+        }
         if (!comm_band(comm, r, pass->rect, &p.rect)) {
             continue;
         }
@@ -2124,7 +2361,7 @@ int rc_gather_device(rc_comm *comm, int which, const rc_rect *rect) {
     rc_ctx *c0 = comm->ctxs[0];
     float4 *dst = const_cast<float4 *>(plane_of(c0, which));
     if (!dst) {
-        return comm_fail(comm, "rc_gather_device: unknown buffer %d", which);
+        return comm_fail(comm, "rc_gather_device: buffer %d does not exist on device %d", which, c0->device);
     }
     if (rc_comm_sync(comm) != 0) {
         return 1;
@@ -2136,6 +2373,9 @@ int rc_gather_device(rc_comm *comm, int which, const rc_rect *rect) {
             continue;
         }
         const float4 *src = plane_of(cr, which);
+        if (!src) {
+            return comm_fail(comm, "rc_gather_device: buffer %d does not exist on device %d", which, cr->device);
+        }
         cudaSetDevice(cr->device);
         cudaMemcpy3DPeerParms pp = {};
         pp.srcDevice = cr->device;
@@ -2264,6 +2504,37 @@ int rc_stage_generate_primary_rays(rc_ctx *ctx, const rc_pass_desc *pass, void *
     const int n_pix_tiles = ((p.rect_w + 7) / 8) * ((p.rect_h + 3) / 4);
     k_raygen<<<(n_pix_tiles * 32 + 255) / 256, 256, 0, ctx->stream>>>(p, ctx->rays[0], ctx->hits);
     CU_CHECK(ctx, cudaStreamSynchronize(ctx->stream));
+    uint32_t n = 0;
+    if (get_counter(ctx, CNT_RAYS + 0, &n)) {
+        return 1;
+    }
+    *count_out = int(n);
+    if (n) {
+        if (download_rays_aos(ctx, ctx->rays[0], static_cast<RayAoS *>(rays_out), int(n)) ||
+            download_hits_aos(ctx, ctx->hits, static_cast<HitAoS *>(hits_out), int(n))) {
+            return 1;
+        }
+    }
+    return 0;
+}
+
+int rc_stage_generate_geo_rays(rc_ctx *ctx, const rc_pass_desc *pass, void *rays_out, void *hits_out, int *count_out) {
+    if (!ctx || !pass || !rays_out || !hits_out || !count_out) {
+        return fail(ctx, "rc_stage_generate_geo_rays: null argument");
+    }
+    if (pass->cam.type != 2) {
+        return fail(ctx, "rc_stage_generate_geo_rays: camera type %u is not Geo (2)", pass->cam.type);
+    }
+    cudaSetDevice(ctx->device);
+    KParams p;
+    if (fill_params(ctx, pass, p) || ensure_geo_lists(ctx, pass)) {
+        return 1;
+    }
+    CU_CHECK(ctx, cudaMemsetAsync(ctx->d_counters, 0, CNT_TOTAL * sizeof(uint32_t), ctx->stream));
+    const int n_pix_tiles = ((p.rect_w + 7) / 8) * ((p.rect_h + 3) / 4);
+    k_raygen_geo<<<(n_pix_tiles * 32 + 255) / 256, 256, 0, ctx->stream>>>(p, geo_params(ctx, pass), ctx->rays[0], ctx->hits);
+    CU_CHECK(ctx, cudaStreamSynchronize(ctx->stream));
+    CU_CHECK(ctx, cudaGetLastError());
     uint32_t n = 0;
     if (get_counter(ctx, CNT_RAYS + 0, &n)) {
         return 1;
@@ -2452,16 +2723,7 @@ void *rc_device_ptr(rc_ctx *ctx, int which) {
     if (!ctx) {
         return nullptr;
     }
-    switch (which) {
-    case RC_BUF_FINAL: return ctx->fb.final;
-    case RC_BUF_RAW: return ctx->fb.raw;
-    case RC_BUF_BASE_COLOR: return ctx->fb.base_color;
-    case RC_BUF_DEPTH_NORMALS: return ctx->fb.depth_normals;
-    case RC_BUF_FULL: return ctx->fb.full;
-    case RC_BUF_HALF: return ctx->fb.half;
-    case RC_BUF_TEMP: return ctx->fb.temp;
-    default: return nullptr;
-    }
+    return const_cast<float4 *>(plane_of(ctx, which));
 }
 
 int rc_event_record(rc_ctx *ctx, int slot) {

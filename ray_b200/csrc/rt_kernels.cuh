@@ -132,6 +132,11 @@ struct FrameBufs {
     int w, h;
 };
 
+// pass flags as k_shade sees them (include/ray_cuda.h RC_RENDER_*): LIGHTING_ONLY acts in the PRIMARY instantiation
+// only; DROP_COL is set on the bounce-1 launch of a SKIP_DIRECT pass.  (NO_BACKGROUND is k_no_background: the
+// test inside k_shade cost the register-capped PRIMARY variants spill stores.)
+enum : uint32_t { KP_LIGHTING_ONLY = 1u, KP_DROP_COL = 4u };
+
 struct KParams {
     ShadeScene sc;
     PassSettings ps;
@@ -148,6 +153,7 @@ struct KParams {
     SortGrid sort_grid;
     uint32_t *sort_keys;
     uint32_t *sort_hist;
+    uint32_t flags; // KP_* (pass flags that reach the shading kernels; set per launch by the host)
 };
 
 RT_DEV RayD load_ray(const RayBuf &b, uint32_t i) {
@@ -372,7 +378,7 @@ __global__ void __launch_bounds__(RT_SHADE_THREADS, RT_SHADE_BLOCKS)
         __syncthreads();
 #endif
         if (more) {
-            shade_surface_b(TEX, c, limit1, out);
+            shade_surface_b(TEX, c, limit1, out, PRIMARY && (p.flags & KP_LIGHTING_ONLY));
         }
         if (valid) {
             const int x = int((xy >> 16) & 0xffff), y = int(xy & 0xffff);
@@ -399,7 +405,7 @@ __global__ void __launch_bounds__(RT_SHADE_THREADS, RT_SHADE_BLOCKS)
                 od.z += (nd.z - od.z) * mix_factor;
                 od.w += (nd.w - od.w) * mix_factor;
                 p.fb.depth_normals[pix] = od;
-            } else {
+            } else if (!(p.flags & KP_DROP_COL)) {
                 float4 o = p.fb.temp[pix];
                 o.x += out.col.x;
                 o.y += out.col.y;
@@ -423,6 +429,18 @@ __global__ void __launch_bounds__(RT_SHADE_THREADS, RT_SHADE_BLOCKS)
         const uint32_t h_slot = warp_append(&p.counters[CNT_SHADOW + bounce], out.has_shadow);
         if (out.has_shadow) {
             store_shadow(out_shadow, h_slot, out.sh_r);
+        }
+    }
+}
+
+// RC_RENDER_NO_BACKGROUND, after the primary shade: camera rays that missed contribute (0,0,0)
+__global__ void k_no_background(KParams p, RayBuf rays, HitBuf hits) {
+    const uint32_t count = p.counters[CNT_RAYS + 0];
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < count; i += gridDim.x * blockDim.x) {
+        if (hits.tuvp[i].z < 0.0f) {
+            const uint32_t xy = rays.xy_depth[i].x;
+            float4 &t = p.fb.temp[int(xy & 0xffff) * p.fb.w + int(xy >> 16)];
+            t.x = t.y = t.z = 0.0f;
         }
     }
 }
@@ -545,8 +563,9 @@ __global__ void __launch_bounds__(256) k_resolve(KParams p, float exposure_mul, 
     }
 }
 
-// add this sample's counters into the persistent 64-bit totals
-__global__ void k_accumulate_totals(KParams p, int max_bounces) {
+// add this sample's counters into the persistent 64-bit totals: the rays of the bounces that were traced, and the
+// shadow rays of the lists in `shadow_traced` (bit b = list b; the pass flags can skip a list)
+__global__ void k_accumulate_totals(KParams p, int max_bounces, uint32_t shadow_traced) {
     if (threadIdx.x == 0 && blockIdx.x == 0) {
         p.totals[TOT_PRIMARY] += p.counters[CNT_RAYS + 0];
         unsigned long long sec = 0, sh = 0;
@@ -554,7 +573,9 @@ __global__ void k_accumulate_totals(KParams p, int max_bounces) {
             sec += p.counters[CNT_RAYS + b];
         }
         for (int b = 0; b <= max_bounces; ++b) {
-            sh += p.counters[CNT_SHADOW + b];
+            if ((shadow_traced >> b) & 1u) {
+                sh += p.counters[CNT_SHADOW + b];
+            }
         }
         p.totals[TOT_SECONDARY] += sec;
         p.totals[TOT_SHADOW] += sh;

@@ -54,6 +54,7 @@ def load_library():
         "rc_reset_stats": (C.c_int, [vp]),
         "rc_get_kernel_ms": (C.c_int, [vp, P(C.c_double), P(C.c_uint64)]),
         "rc_stage_generate_primary_rays": (C.c_int, [vp, P(capi.rc_pass_desc), vp, vp, P(C.c_int)]),
+        "rc_stage_generate_geo_rays": (C.c_int, [vp, P(capi.rc_pass_desc), vp, vp, P(C.c_int)]),
         "rc_stage_trace_rays": (C.c_int, [vp, P(capi.rc_pass_desc), vp, vp, C.c_int, C.c_int]),
         "rc_stage_shade": (C.c_int, [vp, P(capi.rc_pass_desc), C.c_int, C.c_int, vp, vp, C.c_int, vp, P(C.c_int), vp,
                                      P(C.c_int)]),
@@ -97,7 +98,7 @@ EXPORTED_SYMBOLS = [
     "rc_device_count", "rc_create", "rc_destroy", "rc_last_error", "rc_device_name", "rc_resize", "rc_clear",
     "rc_upload_tables", "rc_upload_scene", "rc_render", "rc_denoise_nlm", "rc_sync", "rc_readback", "rc_readback_required_samples",
     "rc_enable_stats", "rc_get_stats", "rc_get_counters", "rc_reset_stats", "rc_get_kernel_ms",
-    "rc_stage_generate_primary_rays", "rc_stage_trace_rays", "rc_stage_shade", "rc_stage_trace_shadow_rays",
+    "rc_stage_generate_primary_rays", "rc_stage_generate_geo_rays", "rc_stage_trace_rays", "rc_stage_shade", "rc_stage_trace_shadow_rays",
     "rc_stage_sort_rays", "rc_debug_fill_temp", "rc_abi_sizeof", "rc_host_alloc", "rc_host_free", "rc_device_ptr",
     "rc_event_record", "rc_event_elapsed_ms", "rc_readback_async", "rc_comm_init", "rc_comm_destroy", "rc_comm_last_error",
     "rc_comm_strip", "rc_comm_upload_scene", "rc_comm_upload_tables", "rc_comm_render", "rc_comm_sync", "rc_gather",
@@ -176,12 +177,15 @@ class Context:
     def scene_upload_bytes(self):
         return int(self.lib.rc_scene_upload_bytes(self._ctx))
 
-    def make_pass(self, cam: capi.rc_camera, rect, iteration, flags=0):
+    def make_pass(self, cam: capi.rc_camera, rect, iteration, flags=0, geo=None):
+        """geo = (instance, tri_first, tri_count): the mesh instance a Geo camera (cam.type == CAM_GEO) bakes."""
         p = capi.rc_pass_desc()
         p.cam = cam
         p.rect = capi.rc_rect(*rect)
         p.iteration = iteration
         p.flags = flags
+        if geo is not None:
+            p.geo_instance, p.geo_tri_first, p.geo_tri_count = (int(x) for x in geo)
         return p
 
     def render(self, p: capi.rc_pass_desc):
@@ -267,6 +271,15 @@ class Context:
         cnt = C.c_int(0)
         self._check(self.lib.rc_stage_generate_primary_rays(self._ctx, C.byref(p), _ptr(rays), _ptr(hits),
                                                             C.byref(cnt)), "rc_stage_generate_primary_rays")
+        return rays[:cnt.value], hits[:cnt.value]
+
+    def stage_generate_geo_rays(self, p):
+        n = p.rect.w * p.rect.h
+        rays = np.zeros(n, dtype=RAY_DTYPE)
+        hits = np.zeros(n, dtype=HIT_DTYPE)
+        cnt = C.c_int(0)
+        self._check(self.lib.rc_stage_generate_geo_rays(self._ctx, C.byref(p), _ptr(rays), _ptr(hits), C.byref(cnt)),
+                    "rc_stage_generate_geo_rays")
         return rays[:cnt.value], hits[:cnt.value]
 
     def stage_trace_rays(self, p, rays, hits, trace_lights):

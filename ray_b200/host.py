@@ -27,7 +27,7 @@ EXPORTED_SYMBOLS = [
     "rh_remove_mesh_instance", "rh_add_light_directional",
     "rh_add_light_sphere", "rh_add_light_spot", "rh_add_light_rect", "rh_add_light_disk", "rh_add_light_line",
     "rh_add_camera", "rh_finalize", "rh_triangle_count", "rh_node_count", "rh_scene_view", "rh_get_camera", "rh_render",
-    "rh_get_pixels", "rh_get_stats", "rh_reset_stats", "rh_get_counters", "rh_get_kernel_ms", "rh_set_sampler_table",
+    "rh_get_pixels", "rh_get_sh_data", "rh_get_stats", "rh_reset_stats", "rh_get_counters", "rh_get_kernel_ms", "rh_set_sampler_table",
     "rh_set_render_flags", "rh_invalidate_scene", "rh_native_context", "rh_builtin_sampler_table", "rh_builtin_filter_table", "rh_abi_sizeof",
 ]
 
@@ -82,6 +82,7 @@ def load_library():
         "rh_get_camera": (None, [vp, P(capi.rc_camera)]),
         "rh_render": (None, [vp, vp, P(capi.rc_rect), P(C.c_int), C.c_int]),
         "rh_get_pixels": (P(C.c_float), [vp, C.c_int, P(C.c_int)]),
+        "rh_get_sh_data": (P(C.c_float), [vp, P(C.c_int)]),
         "rh_get_stats": (None, [vp, P(C.c_uint64)]),
         "rh_reset_stats": (None, [vp]),
         "rh_get_counters": (None, [vp, P(capi.rc_counters)]),
@@ -316,6 +317,16 @@ class Renderer:
         self.check()
         a = np.ctypeslib.as_array(p, shape=(self.hh, pitch.value, 4))[:, :self.w, :]
         return a.copy() if copy else a
+
+    def sh_data(self):
+        """RendererBase::get_sh_data_ref as an (h, w, 3, 4) array (channel r/g/b, 4 L1 coefficients), or None when no
+        pass with camera output_sh has run."""
+        pitch = C.c_int(0)
+        p = self.lib.rh_get_sh_data(self.h, C.byref(pitch))
+        self.check()
+        if not p:
+            return None
+        return np.ctypeslib.as_array(p, shape=(self.hh, pitch.value, 3, 4))[:, :self.w].copy()
 
     def stats_us(self):
         a = (C.c_uint64 * 11)()
