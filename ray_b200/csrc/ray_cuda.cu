@@ -18,6 +18,7 @@
 #include <cuda_runtime.h>
 #include <cub/device/device_scan.cuh>
 
+#include "dev_buf.h"
 #include "rt_kernels.cuh"
 #include "rt_bake.cuh"
 #include "rt_trace.cuh"
@@ -39,9 +40,28 @@ constexpr int kMaxEvents = EV_END + 4;
 enum { KF_RAYGEN = 0, KF_TRACE, KF_SHADE, KF_SHADOW, KF_SORT, KF_RESOLVE, KF_COUNT };
 
 struct DevArray {
-    void *ptr = nullptr;
+    DevBuf<uint8_t> buf;
     size_t bytes = 0;
     uint32_t count = 0;
+
+    void *ptr() const { return buf.get(); }
+    // A non-empty array whose size did not change keeps its block (the common re-upload: animated transforms, edited
+    // materials): a free and a new allocation cost milliseconds and synchronise the device.
+    bool fits(size_t new_bytes) const { return buf.get() && new_bytes != 0 && bytes == new_bytes; }
+    // Sizes the array for `new_bytes` bytes of `new_count` records, contents undefined.  An empty array is a 256-byte
+    // placeholder, so kernels can form (never dereferenced) addresses.
+    cudaError_t resize(size_t new_bytes, uint32_t new_count) {
+        if (!fits(new_bytes)) {
+            bytes = count = 0;
+            const cudaError_t e = buf.alloc(new_bytes ? new_bytes : 256);
+            if (e != cudaSuccess) {
+                return e;
+            }
+        }
+        bytes = new_bytes;
+        count = new_count;
+        return cudaSuccess;
+    }
 };
 
 } // namespace
@@ -55,17 +75,26 @@ struct rc_ctx {
     int num_sms = 0;
 
     int w = 0, h = 0;
+    // fb / rays / hits / shadow are the kernels' views of the per-pixel blocks owned by the DevBufs after them, which
+    // rc_resize allocates
     FrameBufs fb{};
     RayBuf rays[2]{};
     HitBuf hits{};
     ShadowBuf shadow{};
+    DevBuf<float4> fb_planes[7]; // temp, full, half, raw, final, base_color, depth_normals
+    DevBuf<uint16_t> fb_required_samples;
+    DevBuf<float4> ray_planes[2][4]; // o_cw, d_cs, c_pdf, ior of each list
+    DevBuf<uint2> ray_xy_depth[2];
+    DevBuf<float4> hit_tuvp;
+    DevBuf<int> hit_obj;
+    DevBuf<float4> shadow_planes[3]; // o_depth, d_dist, c_xy
     SortBufs sort{};
     size_t ray_capacity = 0;
 
-    uint32_t *d_counters = nullptr;
-    unsigned long long *d_totals = nullptr;
-    uint32_t *d_pmj = nullptr;
-    float *d_filter_table = nullptr;
+    DevBuf<uint32_t> d_counters;
+    DevBuf<unsigned long long> d_totals;
+    DevBuf<uint32_t> d_pmj;
+    DevBuf<float> d_filter_table;
     bool have_tables = false;
 
     DevArray wnodes, mtris, tri_indices, tri_materials, materials, mesh_instances, vertices, vtx_indices, lights,
@@ -75,23 +104,22 @@ struct rc_ctx {
     uint32_t tlas_root_word = kEmptyChild;
     int trace_fin_min = 32;         // lanes of a warp that must have finished before their epilogue + refill is issued
     // UNet denoiser (rt_unet.cuh): weights as uploaded + the 15 intermediate tensors of the current frame size
-    float *unet_w[kUNetLayers] = {}, *unet_b[kUNetLayers] = {};
-    float *unet_t[15] = {};
+    DevBuf<float> unet_w[kUNetLayers], unet_b[kUNetLayers];
+    DevBuf<float> unet_t[15];
     int unet_tw = 0, unet_th = 0; // rounded frame the tensors were sized for
     bool unet_ready = false;
     // tensor-core path (rt_unet_tc.cuh): fp16 weights [9][n][in_cs], fp32 biases [n], bordered fp16 tensors
-    __half *unet_hw[kUNetLayers] = {};
-    float *unet_hb[kUNetLayers] = {};
-    __half *unet_ht[15] = {}, *unet_hx0 = nullptr, *unet_hs = nullptr;
+    DevBuf<__half> unet_hw[kUNetLayers];
+    DevBuf<float> unet_hb[kUNetLayers];
+    DevBuf<__half> unet_ht[15], unet_hx0, unet_hs;
     int unet_htw = 0, unet_hth = 0;
     void *tensor_map_encode = nullptr; // cuTensorMapEncodeTiled through cudaGetDriverEntryPoint
-    float4 *nlm_scratch = nullptr; // 3 planes of the grown region (rt_denoise.cuh)
-    size_t nlm_scratch_elems = 0;
-    uint32_t *d_view_lut[16] = {}; // AgX / Filmic view-transform tables by eViewTransform (rc_set_view_lut)
+    DevBuf<float4> nlm_scratch; // 3 planes of the largest region denoised so far (rt_denoise.cuh)
+    DevBuf<uint32_t> d_view_lut[16]; // AgX / Filmic view-transform tables by eViewTransform (rc_set_view_lut)
     DisplayXf last_xf{nullptr, 1.0f}; // tonemap_params_ of the reference: what the denoisers' display transform uses
     float last_variance_threshold = 0.0f; // tonemap_params_ / variance_threshold_ of the reference
     SceneEnv env{};
-    float *d_srgb_lut = nullptr;
+    DevBuf<float> d_srgb_lut;
     bool have_scene = false;
     rc_scene_view scene_info{};
     uint32_t li_count = 0;
@@ -100,21 +128,19 @@ struct rc_ctx {
     std::map<uint32_t, uint32_t> tex_dense; // (storage << 28 | index) -> dense texture id of the uploaded scene
 
     // Geo camera candidate lists (rt_bake.cuh) of one (scene upload, triangle range, frame size)
-    uint32_t *geo_offsets = nullptr, *geo_cursor = nullptr, *geo_list = nullptr;
-    size_t geo_list_cap = 0;
+    DevBuf<uint32_t> geo_offsets, geo_cursor, geo_list; // geo_list only grows
     bool geo_valid = false;
     uint32_t geo_first = 0, geo_count = 0;
-    // L1 SH planes (RC_BUF_SH_*) + per-sample scratch, allocated by the first RC_RENDER_OUTPUT_SH pass
+    // L1 SH planes (RC_BUF_SH_*) + per-sample scratch, allocated by the first RC_RENDER_OUTPUT_SH pass; `sh` is the
+    // kernels' view of sh_planes
     ShPlanes sh{};
+    DevBuf<float4> sh_planes[7]; // coef[0..2], e0, direct, dir0, dir1
     bool have_sh = false;
     uint32_t sample_tag = 0;
 
     bool stats_enabled = true;
     std::vector<cudaEvent_t> events;
     cudaEvent_t user_events[10] = {}; // 0..7: rc_event_record slots, 8..9: rc_denoise_nlm timing
-    struct PendingSample {
-        int max_bounces;
-    };
     bool sample_pending = false;
     int pending_bounces = 0;
     bool pending_sh = false;
@@ -145,15 +171,11 @@ int fail(rc_ctx *ctx, const char *fmt, ...) {
         }                                                                                                              \
     } while (0)
 
-template <typename T> int dev_alloc(rc_ctx *ctx, T **p, size_t count) {
-    if (*p) {
-        cudaFree(*p);
-        *p = nullptr;
-    }
-    if (count == 0) {
-        return 0;
-    }
-    CU_CHECK(ctx, cudaMalloc(reinterpret_cast<void **>(p), count * sizeof(T)));
+// (Re)allocates `own` for n elements and points the kernel-side view `view` at it (null while it has no block).
+template <typename T> int alloc_view(rc_ctx *ctx, DevBuf<T> &own, T *&view, size_t n) {
+    view = nullptr;
+    CU_CHECK(ctx, own.alloc(n));
+    view = own.get();
     return 0;
 }
 
@@ -165,42 +187,14 @@ int upload_array(rc_ctx *ctx, DevArray &dst, const rc_array &src, uint32_t expec
     if (new_bytes != 0 && !src.ptr) {
         return fail(ctx, "rc_upload_scene: %s has count %u but a null pointer", name, src.count);
     }
-    // a re-upload of an array whose size did not change (the common case: animated transforms, edited materials)
-    // reuses the device allocation: cudaFree + cudaMalloc cost milliseconds and synchronise the device
-    if (!(dst.ptr && new_bytes != 0 && dst.bytes == new_bytes)) {
-        if (dst.ptr) {
-            cudaFree(dst.ptr);
-            dst = DevArray{};
-        }
-        CU_CHECK(ctx, cudaMalloc(&dst.ptr, new_bytes ? new_bytes : 256));
-    }
-    dst.count = src.count;
-    dst.bytes = new_bytes;
+    CU_CHECK(ctx, dst.resize(new_bytes, src.count));
     if (new_bytes == 0) {
-        // a valid non-null pointer so kernels can form (never dereferenced) addresses
-        CU_CHECK(ctx, cudaMemsetAsync(dst.ptr, 0, 256, ctx->stream));
+        CU_CHECK(ctx, cudaMemsetAsync(dst.ptr(), 0, 256, ctx->stream));
         return 0;
     }
-    CU_CHECK(ctx, cudaMemcpyAsync(dst.ptr, src.ptr, dst.bytes, cudaMemcpyHostToDevice, ctx->stream));
+    CU_CHECK(ctx, cudaMemcpyAsync(dst.ptr(), src.ptr, dst.bytes, cudaMemcpyHostToDevice, ctx->stream));
     ctx->scene_h2d_bytes += dst.bytes;
     return 0;
-}
-
-int alloc_ray_buf(rc_ctx *ctx, RayBuf &b, size_t n) {
-    if (dev_alloc(ctx, &b.o_cw, n) || dev_alloc(ctx, &b.d_cs, n) || dev_alloc(ctx, &b.c_pdf, n) ||
-        dev_alloc(ctx, &b.ior, n) || dev_alloc(ctx, &b.xy_depth, n)) {
-        return 1;
-    }
-    return 0;
-}
-
-void free_ray_buf(RayBuf &b) {
-    cudaFree(b.o_cw);
-    cudaFree(b.d_cs);
-    cudaFree(b.c_pdf);
-    cudaFree(b.ior);
-    cudaFree(b.xy_depth);
-    b = RayBuf{};
 }
 
 // murmur3 finaliser on the host (reference CoreRef.h:133-141) for rand_seed = hash((iteration - 1) / 4096)
@@ -249,10 +243,10 @@ int fill_params(rc_ctx *ctx, const rc_pass_desc *pass, KParams &p) {
             return fail(ctx, "Geo camera: a %dx%d lightmap has more than 2^31 texels", ctx->w, ctx->h);
         }
     }
-    if (c.view_transform != 0 && (c.view_transform >= 16 || !ctx->d_view_lut[c.view_transform])) {
+    if (c.view_transform != 0 && (c.view_transform >= 16 || !ctx->d_view_lut[c.view_transform].get())) {
         return fail(ctx, "view transform %u needs its table (rc_set_view_lut)", c.view_transform);
     }
-    if (c.filter != 0 && !ctx->d_filter_table) {
+    if (c.filter != 0 && !ctx->d_filter_table.get()) {
         return fail(ctx, "pixel filter %u needs a filter table (rc_upload_tables)", c.filter);
     }
     if (c.max_total_depth + 1 >= uint32_t(kMaxBounces)) {
@@ -267,26 +261,26 @@ int fill_params(rc_ctx *ctx, const rc_pass_desc *pass, KParams &p) {
     }
 
     memset(&p, 0, sizeof(p));
-    p.sc.geo.nodes = static_cast<const WNode *>(ctx->wnodes.ptr);
-    p.sc.geo.dnodes = static_cast<const WNode *>(ctx->dnodes.ptr);
-    p.sc.geo.blas_roots = static_cast<const uint32_t *>(ctx->blas_roots.ptr);
-    p.sc.geo.dmtris = ctx->dmtris.ptr;
+    p.sc.geo.nodes = static_cast<const WNode *>(ctx->wnodes.ptr());
+    p.sc.geo.dnodes = static_cast<const WNode *>(ctx->dnodes.ptr());
+    p.sc.geo.blas_roots = static_cast<const uint32_t *>(ctx->blas_roots.ptr());
+    p.sc.geo.dmtris = ctx->dmtris.ptr();
     p.sc.geo.tlas_root_word = ctx->tlas_root_word;
-    p.sc.geo.mtris = static_cast<const MTri *>(ctx->mtris.ptr);
-    p.sc.geo.tri_indices = static_cast<const uint32_t *>(ctx->tri_indices.ptr);
-    p.sc.geo.tri_materials = static_cast<const TriMat *>(ctx->tri_materials.ptr);
-    p.sc.geo.instances = static_cast<const MeshInstance *>(ctx->mesh_instances.ptr);
+    p.sc.geo.mtris = static_cast<const MTri *>(ctx->mtris.ptr());
+    p.sc.geo.tri_indices = static_cast<const uint32_t *>(ctx->tri_indices.ptr());
+    p.sc.geo.tri_materials = static_cast<const TriMat *>(ctx->tri_materials.ptr());
+    p.sc.geo.instances = static_cast<const MeshInstance *>(ctx->mesh_instances.ptr());
     p.sc.geo.tlas_root = ctx->scene_info.tlas_root;
-    p.sc.surf.vertices = static_cast<const Vertex *>(ctx->vertices.ptr);
-    p.sc.surf.vtx_indices = static_cast<const uint32_t *>(ctx->vtx_indices.ptr);
-    p.sc.surf.materials = static_cast<const Material *>(ctx->materials.ptr);
-    p.sc.tex.descs = ctx->tex_descs.count ? static_cast<const TexDesc *>(ctx->tex_descs.ptr) : nullptr;
-    p.sc.tex.texels = static_cast<const uint32_t *>(ctx->tex_texels.ptr);
-    p.sc.tex.srgb_lut = ctx->d_srgb_lut;
+    p.sc.surf.vertices = static_cast<const Vertex *>(ctx->vertices.ptr());
+    p.sc.surf.vtx_indices = static_cast<const uint32_t *>(ctx->vtx_indices.ptr());
+    p.sc.surf.materials = static_cast<const Material *>(ctx->materials.ptr());
+    p.sc.tex.descs = ctx->tex_descs.count ? static_cast<const TexDesc *>(ctx->tex_descs.ptr()) : nullptr;
+    p.sc.tex.texels = static_cast<const uint32_t *>(ctx->tex_texels.ptr());
+    p.sc.tex.srgb_lut = ctx->d_srgb_lut.get();
     p.sc.lights.env = ctx->env;
-    p.sc.lights.env.qtree = static_cast<const float4 *>(ctx->qtree.ptr);
-    p.sc.lights.lights = static_cast<const Light *>(ctx->lights.ptr);
-    p.sc.lights.nodes = static_cast<const LightCWNode *>(ctx->light_cwnodes.ptr);
+    p.sc.lights.env.qtree = static_cast<const float4 *>(ctx->qtree.ptr());
+    p.sc.lights.lights = static_cast<const Light *>(ctx->lights.ptr());
+    p.sc.lights.nodes = static_cast<const LightCWNode *>(ctx->light_cwnodes.ptr());
     p.sc.lights.nodes_count = ctx->light_cwnodes.count;
     p.sc.lights.visible_lights_count = ctx->scene_info.visible_lights_count;
     p.sc.lights.blocker_lights_count = ctx->scene_info.blocker_lights_count;
@@ -295,7 +289,7 @@ int fill_params(rc_ctx *ctx, const rc_pass_desc *pass, KParams &p) {
         p.sc.lights.env_col[i] = ctx->scene_info.env_col[i];
         p.sc.lights.back_col[i] = ctx->scene_info.back_col[i];
     }
-    p.sc.rand_seq = ctx->d_pmj;
+    p.sc.rand_seq = ctx->d_pmj.get();
     p.sc.li_count = ctx->li_count;
 
     p.ps.max_diff_depth = int(c.max_diff_depth);
@@ -333,9 +327,9 @@ int fill_params(rc_ctx *ctx, const rc_pass_desc *pass, KParams &p) {
     p.cam.filter = int(c.filter);
 
     p.fb = ctx->fb;
-    p.filter_table = ctx->d_filter_table;
-    p.counters = ctx->d_counters;
-    p.totals = ctx->d_totals;
+    p.filter_table = ctx->d_filter_table.get();
+    p.counters = ctx->d_counters.get();
+    p.totals = ctx->d_totals.get();
     p.rect_x = r.x;
     p.rect_y = r.y;
     p.rect_w = r.w;
@@ -414,24 +408,12 @@ int validate_bvh(rc_ctx *ctx, const rc_scene_view *sv) {
 int build_traversal_copies(rc_ctx *ctx, const rc_scene_view *sv) {
     const uint32_t n_nodes = sv->wnodes.count, n_inst = sv->mesh_instances.count;
     const uint32_t n_blocks = sv->mtris.count;
-    for (DevArray *a : {&ctx->dnodes, &ctx->blas_roots, &ctx->dmtris}) {
-        const size_t want = (a == &ctx->dnodes) ? size_t(n_nodes) * sizeof(WNode)
-                                                : (a == &ctx->dmtris ? size_t(n_blocks) * sizeof(MTri) : size_t(n_inst) * 4);
-        if (!(a->ptr && want != 0 && a->bytes == want)) {
-            if (a->ptr) {
-                cudaFree(a->ptr);
-                *a = DevArray{};
-            }
-            CU_CHECK(ctx, cudaMalloc(&a->ptr, want ? want : 256));
-        }
-        a->bytes = want;
-    }
-    ctx->dnodes.count = n_nodes;
-    ctx->blas_roots.count = n_inst;
-    ctx->dmtris.count = n_blocks;
+    CU_CHECK(ctx, ctx->dnodes.resize(size_t(n_nodes) * sizeof(WNode), n_nodes));
+    CU_CHECK(ctx, ctx->blas_roots.resize(size_t(n_inst) * 4, n_inst));
+    CU_CHECK(ctx, ctx->dmtris.resize(size_t(n_blocks) * sizeof(MTri), n_blocks));
     if (n_blocks != 0) {
-        k_build_dmtris<<<(n_blocks * 4 + 255) / 256, 256, 0, ctx->stream>>>(static_cast<const MTri *>(ctx->mtris.ptr),
-                                                                          static_cast<float4 *>(ctx->dmtris.ptr), n_blocks);
+        k_build_dmtris<<<(n_blocks * 4 + 255) / 256, 256, 0, ctx->stream>>>(static_cast<const MTri *>(ctx->mtris.ptr()),
+                                                                          static_cast<float4 *>(ctx->dmtris.ptr()), n_blocks);
     }
     ctx->tlas_root_word = kEmptyChild;
     if (validate_bvh(ctx, sv)) {
@@ -439,12 +421,12 @@ int build_traversal_copies(rc_ctx *ctx, const rc_scene_view *sv) {
     }
     if (n_nodes != 0) {
         k_build_dnodes<<<(n_nodes * 8 + 255) / 256, 256, 0, ctx->stream>>>(
-            static_cast<const WNode *>(ctx->wnodes.ptr), static_cast<WNode *>(ctx->dnodes.ptr), 0u, n_nodes);
+            static_cast<const WNode *>(ctx->wnodes.ptr()), static_cast<WNode *>(ctx->dnodes.ptr()), 0u, n_nodes);
     }
     if (n_inst != 0) {
         k_build_blas_roots<<<(n_inst + 255) / 256, 256, 0, ctx->stream>>>(
-            static_cast<const WNode *>(ctx->wnodes.ptr), static_cast<const MeshInstance *>(ctx->mesh_instances.ptr), n_inst,
-            n_nodes, static_cast<uint32_t *>(ctx->blas_roots.ptr));
+            static_cast<const WNode *>(ctx->wnodes.ptr()), static_cast<const MeshInstance *>(ctx->mesh_instances.ptr()), n_inst,
+            n_nodes, static_cast<uint32_t *>(ctx->blas_roots.ptr()));
     }
     CU_CHECK(ctx, cudaStreamSynchronize(ctx->stream));
     CU_CHECK(ctx, cudaGetLastError());
@@ -480,7 +462,7 @@ const float4 *plane_of(const rc_ctx *ctx, int which) {
     case RC_BUF_TEMP: return ctx->fb.temp;
     case RC_BUF_SH_R:
     case RC_BUF_SH_G:
-    case RC_BUF_SH_B: return ctx->sh.coef[which - RC_BUF_SH_R];
+    case RC_BUF_SH_B: return ctx->have_sh ? ctx->sh.coef[which - RC_BUF_SH_R] : nullptr;
     default: return nullptr;
     }
 }
@@ -582,17 +564,8 @@ void launch_shade(rc_ctx *ctx, int grid, cudaStream_t s, const KParams &p, RayBu
 }
 
 GeoTarget geo_target(const rc_ctx *ctx, const rc_pass_desc *pass) {
-    return GeoTarget{static_cast<const Vertex *>(ctx->vertices.ptr), static_cast<const uint32_t *>(ctx->vtx_indices.ptr),
+    return GeoTarget{static_cast<const Vertex *>(ctx->vertices.ptr()), static_cast<const uint32_t *>(ctx->vtx_indices.ptr()),
                      pass->geo_tri_first, pass->geo_tri_count, ctx->w, ctx->h};
-}
-
-void free_geo_lists(rc_ctx *ctx) {
-    cudaFree(ctx->geo_offsets);
-    cudaFree(ctx->geo_cursor);
-    cudaFree(ctx->geo_list);
-    ctx->geo_offsets = ctx->geo_cursor = ctx->geo_list = nullptr;
-    ctx->geo_list_cap = 0;
-    ctx->geo_valid = false;
 }
 
 // Build (or reuse) the per-texel candidate lists of a Geo pass (rt_bake.cuh).  Blocking when it builds.
@@ -604,51 +577,51 @@ int ensure_geo_lists(rc_ctx *ctx, const rc_pass_desc *pass) {
     cudaStream_t s = ctx->stream;
     const GeoTarget g = geo_target(ctx, pass);
     const size_t n = size_t(ctx->w) * ctx->h;
-    if (!ctx->geo_offsets) {
-        if (dev_alloc(ctx, &ctx->geo_offsets, n + 1) || dev_alloc(ctx, &ctx->geo_cursor, n + 1)) {
-            return 1;
-        }
+    if (!ctx->geo_offsets.get()) {
+        CU_CHECK(ctx, ctx->geo_offsets.alloc(n + 1));
+        CU_CHECK(ctx, ctx->geo_cursor.alloc(n + 1));
     }
-    unsigned long long *d_total = nullptr, total = 0;
-    CU_CHECK(ctx, cudaMalloc(&d_total, sizeof(*d_total)));
-    cudaMemsetAsync(d_total, 0, sizeof(*d_total), s);
     const uint32_t tris = g.tri_count;
-    if (tris != 0) {
-        k_geo_box_total<<<(tris + 255) / 256, 256, 0, s>>>(g, d_total);
+    unsigned long long total = 0;
+    {
+        DevBuf<unsigned long long> d_total;
+        CU_CHECK(ctx, d_total.alloc(1));
+        cudaMemsetAsync(d_total.get(), 0, sizeof(total), s);
+        if (tris != 0) {
+            k_geo_box_total<<<(tris + 255) / 256, 256, 0, s>>>(g, d_total.get());
+        }
+        const cudaError_t e = cudaMemcpyAsync(&total, d_total.get(), sizeof(total), cudaMemcpyDeviceToHost, s);
+        cudaStreamSynchronize(s);
+        CU_CHECK(ctx, e);
     }
-    const cudaError_t e = cudaMemcpyAsync(&total, d_total, sizeof(total), cudaMemcpyDeviceToHost, s);
-    cudaStreamSynchronize(s);
-    cudaFree(d_total);
-    CU_CHECK(ctx, e);
     CU_CHECK(ctx, cudaGetLastError());
     if (total > kGeoMaxEntries) {
         return fail(ctx, "Geo camera: the candidate lists of triangles [%u, %u) at %dx%d would hold %llu entries, more than "
                          "the 2^28 (1 GiB) the backend allows",
                     g.tri_first, g.tri_first + g.tri_count, ctx->w, ctx->h, total);
     }
-    if (total > ctx->geo_list_cap || !ctx->geo_list) {
-        if (dev_alloc(ctx, &ctx->geo_list, size_t(total ? total : 1))) {
-            return 1;
-        }
-        ctx->geo_list_cap = size_t(total);
+    if (!ctx->geo_list.get() || total > ctx->geo_list.count()) {
+        CU_CHECK(ctx, ctx->geo_list.alloc(size_t(total ? total : 1)));
     }
-    CU_CHECK(ctx, cudaMemsetAsync(ctx->geo_cursor, 0, (n + 1) * sizeof(uint32_t), s));
+    CU_CHECK(ctx, cudaMemsetAsync(ctx->geo_cursor.get(), 0, (n + 1) * sizeof(uint32_t), s));
     const int warp_blocks = int(std::min<uint64_t>((uint64_t(tris) * 32 + 255) / 256, uint64_t(ctx->num_sms) * 64));
     if (tris != 0) {
-        k_geo_walk<false><<<warp_blocks, 256, 0, s>>>(g, ctx->geo_cursor, nullptr);
+        k_geo_walk<false><<<warp_blocks, 256, 0, s>>>(g, ctx->geo_cursor.get(), nullptr);
     }
-    size_t temp_bytes = 0;
-    cub::DeviceScan::ExclusiveSum(nullptr, temp_bytes, ctx->geo_cursor, ctx->geo_offsets, int(n + 1), s);
-    void *d_temp = nullptr;
-    CU_CHECK(ctx, cudaMalloc(&d_temp, temp_bytes ? temp_bytes : 16));
-    cub::DeviceScan::ExclusiveSum(d_temp, temp_bytes, ctx->geo_cursor, ctx->geo_offsets, int(n + 1), s);
-    const cudaError_t e2 = cudaMemcpyAsync(ctx->geo_cursor, ctx->geo_offsets, n * sizeof(uint32_t), cudaMemcpyDeviceToDevice, s);
-    if (e2 == cudaSuccess && tris != 0) {
-        k_geo_walk<true><<<warp_blocks, 256, 0, s>>>(g, ctx->geo_cursor, ctx->geo_list);
+    {
+        size_t temp_bytes = 0;
+        cub::DeviceScan::ExclusiveSum(nullptr, temp_bytes, ctx->geo_cursor.get(), ctx->geo_offsets.get(), int(n + 1), s);
+        DevBuf<uint8_t> d_temp;
+        CU_CHECK(ctx, d_temp.alloc(temp_bytes ? temp_bytes : 16));
+        cub::DeviceScan::ExclusiveSum(d_temp.get(), temp_bytes, ctx->geo_cursor.get(), ctx->geo_offsets.get(), int(n + 1), s);
+        const cudaError_t e = cudaMemcpyAsync(ctx->geo_cursor.get(), ctx->geo_offsets.get(), n * sizeof(uint32_t),
+                                              cudaMemcpyDeviceToDevice, s);
+        if (e == cudaSuccess && tris != 0) {
+            k_geo_walk<true><<<warp_blocks, 256, 0, s>>>(g, ctx->geo_cursor.get(), ctx->geo_list.get());
+        }
+        cudaStreamSynchronize(s);
+        CU_CHECK(ctx, e);
     }
-    cudaStreamSynchronize(s);
-    cudaFree(d_temp);
-    CU_CHECK(ctx, e2);
     CU_CHECK(ctx, cudaGetLastError());
     ctx->geo_first = pass->geo_tri_first;
     ctx->geo_count = pass->geo_tri_count;
@@ -657,29 +630,20 @@ int ensure_geo_lists(rc_ctx *ctx, const rc_pass_desc *pass) {
 }
 
 GeoParams geo_params(const rc_ctx *ctx, const rc_pass_desc *pass) {
-    return GeoParams{geo_target(ctx, pass), ctx->geo_offsets, ctx->geo_list,
-                     static_cast<const MeshInstance *>(ctx->mesh_instances.ptr) + pass->geo_instance, pass->geo_instance};
-}
-
-void free_sh(rc_ctx *ctx) {
-    for (float4 *b : {ctx->sh.coef[0], ctx->sh.coef[1], ctx->sh.coef[2], ctx->sh.e0, ctx->sh.direct, ctx->sh.dir0, ctx->sh.dir1}) {
-        cudaFree(b);
-    }
-    ctx->sh = ShPlanes{};
-    ctx->have_sh = false;
+    return GeoParams{geo_target(ctx, pass), ctx->geo_offsets.get(), ctx->geo_list.get(),
+                     static_cast<const MeshInstance *>(ctx->mesh_instances.ptr()) + pass->geo_instance, pass->geo_instance};
 }
 
 // the SH planes (zeroed) + scratch at the current frame size
 int alloc_sh(rc_ctx *ctx) {
     const size_t n = size_t(ctx->w) * ctx->h;
-    free_sh(ctx);
-    for (float4 **b : {&ctx->sh.coef[0], &ctx->sh.coef[1], &ctx->sh.coef[2], &ctx->sh.e0, &ctx->sh.direct, &ctx->sh.dir0,
-                       &ctx->sh.dir1}) {
-        if (dev_alloc(ctx, b, n)) {
-            free_sh(ctx);
+    ShPlanes &sh = ctx->sh;
+    float4 **views[7] = {&sh.coef[0], &sh.coef[1], &sh.coef[2], &sh.e0, &sh.direct, &sh.dir0, &sh.dir1};
+    for (int i = 0; i < 7; ++i) {
+        if (alloc_view(ctx, ctx->sh_planes[i], *views[i], n)) {
             return 1;
         }
-        CU_CHECK(ctx, cudaMemsetAsync(*b, 0, n * sizeof(float4), ctx->stream));
+        CU_CHECK(ctx, cudaMemsetAsync(*views[i], 0, n * sizeof(float4), ctx->stream));
     }
     ctx->have_sh = true;
     return 0;
@@ -711,14 +675,14 @@ int enqueue_sample(rc_ctx *ctx, const rc_pass_desc *pass, KParams &p) {
         harvest_stats(ctx);
     }
 
-    CU_CHECK(ctx, cudaMemsetAsync(ctx->d_counters, 0, CNT_TOTAL * sizeof(uint32_t), s));
+    CU_CHECK(ctx, cudaMemsetAsync(ctx->d_counters.get(), 0, CNT_TOTAL * sizeof(uint32_t), s));
     if (do_sort) {
         // k_shade emits sort keys + per-list histograms while it writes the secondary rays
-        CU_CHECK(ctx, cudaMemsetAsync(ctx->sort.hist, 0, size_t(max_bounces + 2) * kSortBins * sizeof(uint32_t), s));
+        CU_CHECK(ctx, cudaMemsetAsync(ctx->sort.hist.get(), 0, size_t(max_bounces + 2) * kSortBins * sizeof(uint32_t), s));
         p.sort_grid = SortGrid{ctx->sort.root_min[0], ctx->sort.root_min[1], ctx->sort.root_min[2],
                                ctx->sort.inv_cell[0], ctx->sort.inv_cell[1], ctx->sort.inv_cell[2]};
-        p.sort_keys = ctx->sort.keys;
-        p.sort_hist = ctx->sort.hist;
+        p.sort_keys = ctx->sort.keys.get();
+        p.sort_hist = ctx->sort.hist.get();
     }
     record(ctx, EV_START);
 
@@ -820,7 +784,7 @@ int enqueue_sample(rc_ctx *ctx, const rc_pass_desc *pass, KParams &p) {
         const float vt = p.iteration > pass->cam.min_samples
                              ? 0.5f * pass->cam.variance_threshold * pass->cam.variance_threshold
                              : 0.0f;
-        const DisplayXf xf{pass->cam.view_transform ? ctx->d_view_lut[pass->cam.view_transform] : nullptr, inv_gamma};
+        const DisplayXf xf{pass->cam.view_transform ? ctx->d_view_lut[pass->cam.view_transform].get() : nullptr, inv_gamma};
         if (want_sh) { // reads temp before k_resolve overwrites it with the variance
             k_sh_resolve<<<(n_rect + 255) / 256, 256, 0, s>>>(p, ctx->sh, tag, exposure_mul, mix_factor);
             ctx->kernel_launches[KF_RESOLVE]++;
@@ -937,12 +901,12 @@ int download_shadow_aos(rc_ctx *ctx, const ShadowBuf &b, ShadowRayAoS *dst, int 
 }
 
 int set_counter(rc_ctx *ctx, int slot, uint32_t v) {
-    CU_CHECK(ctx, cudaMemcpy(ctx->d_counters + slot, &v, sizeof(v), cudaMemcpyHostToDevice));
+    CU_CHECK(ctx, cudaMemcpy(ctx->d_counters.get() + slot, &v, sizeof(v), cudaMemcpyHostToDevice));
     return 0;
 }
 
 int get_counter(rc_ctx *ctx, int slot, uint32_t *v) {
-    CU_CHECK(ctx, cudaMemcpy(v, ctx->d_counters + slot, sizeof(*v), cudaMemcpyDeviceToHost));
+    CU_CHECK(ctx, cudaMemcpy(v, ctx->d_counters.get() + slot, sizeof(*v), cudaMemcpyDeviceToHost));
     return 0;
 }
 
@@ -982,6 +946,25 @@ int rc_create(int device, rc_ctx **out_ctx) {
     }
     ctx->device_name = ctx->prop.name;
     ctx->num_sms = ctx->prop.multiProcessorCount;
+    // every failure below returns through `delete ctx`: what was allocated so far frees itself, with the device current
+    if (ctx->d_counters.alloc(CNT_TOTAL) != cudaSuccess || ctx->d_totals.alloc(TOT_COUNT) != cudaSuccess) {
+        delete ctx;
+        return 6;
+    }
+    cudaMemset(ctx->d_counters.get(), 0, CNT_TOTAL * sizeof(uint32_t));
+    cudaMemset(ctx->d_totals.get(), 0, TOT_COUNT * sizeof(unsigned long long));
+    { // srgb_to_linear (CoreRef.h:208-220) of the 256 values a texel channel can hold, with the HOST powf like the reference
+        float lut[256];
+        for (int i = 0; i < 256; ++i) {
+            const float c = float(i) / 255.0f;
+            lut[i] = (c > 0.04045f) ? powf((c + 0.055f) / 1.055f, 2.4f) : (c / 12.92f);
+        }
+        if (ctx->d_srgb_lut.alloc(256) != cudaSuccess ||
+            cudaMemcpy(ctx->d_srgb_lut.get(), lut, sizeof(lut), cudaMemcpyHostToDevice) != cudaSuccess) {
+            delete ctx;
+            return 6;
+        }
+    }
     if (cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking) != cudaSuccess) {
         delete ctx;
         return 5;
@@ -992,24 +975,6 @@ int rc_create(int device, rc_ctx **out_ctx) {
     }
     for (auto &e : ctx->user_events) {
         cudaEventCreate(&e);
-    }
-    if (dev_alloc(ctx, &ctx->d_counters, CNT_TOTAL) || dev_alloc(ctx, &ctx->d_totals, TOT_COUNT)) {
-        rc_destroy(ctx);
-        return 6;
-    }
-    cudaMemset(ctx->d_counters, 0, CNT_TOTAL * sizeof(uint32_t));
-    cudaMemset(ctx->d_totals, 0, TOT_COUNT * sizeof(unsigned long long));
-    { // srgb_to_linear (CoreRef.h:208-220) of the 256 values a texel channel can hold, with the HOST powf like the reference
-        float lut[256];
-        for (int i = 0; i < 256; ++i) {
-            const float c = float(i) / 255.0f;
-            lut[i] = (c > 0.04045f) ? powf((c + 0.055f) / 1.055f, 2.4f) : (c / 12.92f);
-        }
-        if (cudaMalloc(&ctx->d_srgb_lut, sizeof(lut)) != cudaSuccess ||
-            cudaMemcpy(ctx->d_srgb_lut, lut, sizeof(lut), cudaMemcpyHostToDevice) != cudaSuccess) {
-            rc_destroy(ctx);
-            return 6;
-        }
     }
     // the trace kernels keep their stacks in static shared memory (rt_trace.cuh): RT_TRACE_BLOCKS blocks must fit, the
     // rest of the unified array stays L1
@@ -1029,6 +994,8 @@ int rc_create(int device, rc_ctx **out_ctx) {
     cudaFuncSetAttribute(k_shade<false, false>, cudaFuncAttributePreferredSharedMemoryCarveout, 0);
     cudaFuncSetAttribute(k_shade<true, true>, cudaFuncAttributePreferredSharedMemoryCarveout, 0);
     cudaFuncSetAttribute(k_shade<false, true>, cudaFuncAttributePreferredSharedMemoryCarveout, 0);
+    // function attributes apply to the current device: each context sets them for its own
+    cudaFuncSetAttribute(tc::k_unet_conv_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::kSmemBudget + 1024);
     *out_ctx = ctx;
     return 0;
 }
@@ -1037,68 +1004,15 @@ void rc_destroy(rc_ctx *ctx) {
     if (!ctx) {
         return;
     }
-    cudaSetDevice(ctx->device);
-    if (ctx->stream) {
-        cudaStreamSynchronize(ctx->stream);
-    }
+    cudaSetDevice(ctx->device); // the members' destructors free their blocks on this device
+    cudaStreamSynchronize(ctx->stream);
     for (auto &e : ctx->events) {
         cudaEventDestroy(e);
     }
     for (auto &e : ctx->user_events) {
         cudaEventDestroy(e);
     }
-    for (uint32_t *&l : ctx->d_view_lut) {
-        cudaFree(l);
-        l = nullptr;
-    }
-    cudaFree(ctx->fb.temp);
-    cudaFree(ctx->fb.full);
-    cudaFree(ctx->fb.half);
-    cudaFree(ctx->fb.raw);
-    cudaFree(ctx->fb.final);
-    cudaFree(ctx->fb.base_color);
-    cudaFree(ctx->fb.depth_normals);
-    cudaFree(ctx->fb.required_samples);
-    free_ray_buf(ctx->rays[0]);
-    free_ray_buf(ctx->rays[1]);
-    cudaFree(ctx->hits.tuvp);
-    cudaFree(ctx->hits.obj);
-    cudaFree(ctx->shadow.o_depth);
-    cudaFree(ctx->shadow.d_dist);
-    cudaFree(ctx->shadow.c_xy);
-    free_sort_bufs(ctx->sort);
-    cudaFree(ctx->d_counters);
-    cudaFree(ctx->d_totals);
-    cudaFree(ctx->d_pmj);
-    cudaFree(ctx->d_filter_table);
-    cudaFree(ctx->d_srgb_lut);
-    cudaFree(ctx->nlm_scratch);
-    free_geo_lists(ctx);
-    free_sh(ctx);
-    for (int i = 0; i < kUNetLayers; ++i) {
-        cudaFree(ctx->unet_w[i]);
-        cudaFree(ctx->unet_b[i]);
-    }
-    for (float *t : ctx->unet_t) {
-        cudaFree(t);
-    }
-    for (int i = 0; i < kUNetLayers; ++i) {
-        cudaFree(ctx->unet_hw[i]);
-        cudaFree(ctx->unet_hb[i]);
-    }
-    for (__half *t : ctx->unet_ht) {
-        cudaFree(t);
-    }
-    cudaFree(ctx->unet_hx0);
-    cudaFree(ctx->unet_hs);
-    for (DevArray *a : {&ctx->dnodes, &ctx->blas_roots, &ctx->dmtris, &ctx->wnodes, &ctx->mtris, &ctx->tri_indices, &ctx->tri_materials, &ctx->materials,
-                        &ctx->mesh_instances, &ctx->vertices, &ctx->vtx_indices, &ctx->lights, &ctx->light_cwnodes,
-                        &ctx->tex_descs, &ctx->tex_texels, &ctx->qtree}) {
-        cudaFree(a->ptr);
-    }
-    if (ctx->stream) {
-        cudaStreamDestroy(ctx->stream);
-    }
+    cudaStreamDestroy(ctx->stream);
     delete ctx;
 }
 
@@ -1119,29 +1033,54 @@ int rc_resize(rc_ctx *ctx, int w, int h) {
     // for a zero-size frame), not pointing at freed or mis-sized planes
     ctx->w = ctx->h = ctx->fb.w = ctx->fb.h = 0;
     ctx->ray_capacity = 0;
-    free_geo_lists(ctx);
+    ctx->geo_offsets.reset();
+    ctx->geo_cursor.reset();
+    ctx->geo_list.reset();
+    ctx->geo_valid = false;
     const bool had_sh = ctx->have_sh;
-    free_sh(ctx);
-    if (dev_alloc(ctx, &ctx->fb.temp, n) || dev_alloc(ctx, &ctx->fb.full, n) || dev_alloc(ctx, &ctx->fb.half, n) ||
-        dev_alloc(ctx, &ctx->fb.raw, n) || dev_alloc(ctx, &ctx->fb.final, n) || dev_alloc(ctx, &ctx->fb.base_color, n) ||
-        dev_alloc(ctx, &ctx->fb.depth_normals, n) || dev_alloc(ctx, &ctx->fb.required_samples, n)) {
+    ctx->have_sh = false;
+    for (DevBuf<float4> &b : ctx->sh_planes) {
+        b.reset();
+    }
+    FrameBufs &fb = ctx->fb;
+    float4 **planes[7] = {&fb.temp, &fb.full, &fb.half, &fb.raw, &fb.final, &fb.base_color, &fb.depth_normals};
+    for (int i = 0; i < 7; ++i) {
+        if (alloc_view(ctx, ctx->fb_planes[i], *planes[i], n)) {
+            return 1;
+        }
+    }
+    if (alloc_view(ctx, ctx->fb_required_samples, fb.required_samples, n)) {
         return 1;
     }
     if (n) {
-        for (float4 *b : {ctx->fb.temp, ctx->fb.full, ctx->fb.half, ctx->fb.raw, ctx->fb.final, ctx->fb.base_color,
-                          ctx->fb.depth_normals}) {
-            CU_CHECK(ctx, cudaMemsetAsync(b, 0, n * sizeof(float4), ctx->stream));
+        for (float4 **b : planes) {
+            CU_CHECK(ctx, cudaMemsetAsync(*b, 0, n * sizeof(float4), ctx->stream));
         }
-        CU_CHECK(ctx, cudaMemsetAsync(ctx->fb.required_samples, 0xff, n * sizeof(uint16_t), ctx->stream));
+        CU_CHECK(ctx, cudaMemsetAsync(fb.required_samples, 0xff, n * sizeof(uint16_t), ctx->stream));
     }
-    if (alloc_ray_buf(ctx, ctx->rays[0], n) || alloc_ray_buf(ctx, ctx->rays[1], n) || dev_alloc(ctx, &ctx->hits.tuvp, n) ||
-        dev_alloc(ctx, &ctx->hits.obj, n) || dev_alloc(ctx, &ctx->shadow.o_depth, n) ||
-        dev_alloc(ctx, &ctx->shadow.d_dist, n) || dev_alloc(ctx, &ctx->shadow.c_xy, n)) {
+    for (int l = 0; l < 2; ++l) {
+        RayBuf &r = ctx->rays[l];
+        if (alloc_view(ctx, ctx->ray_planes[l][0], r.o_cw, n) || alloc_view(ctx, ctx->ray_planes[l][1], r.d_cs, n) ||
+            alloc_view(ctx, ctx->ray_planes[l][2], r.c_pdf, n) || alloc_view(ctx, ctx->ray_planes[l][3], r.ior, n) ||
+            alloc_view(ctx, ctx->ray_xy_depth[l], r.xy_depth, n)) {
+            return 1;
+        }
+    }
+    if (alloc_view(ctx, ctx->hit_tuvp, ctx->hits.tuvp, n) || alloc_view(ctx, ctx->hit_obj, ctx->hits.obj, n) ||
+        alloc_view(ctx, ctx->shadow_planes[0], ctx->shadow.o_depth, n) ||
+        alloc_view(ctx, ctx->shadow_planes[1], ctx->shadow.d_dist, n) ||
+        alloc_view(ctx, ctx->shadow_planes[2], ctx->shadow.c_xy, n)) {
         return 1;
     }
-    if (alloc_sort_bufs(ctx->sort, n) != 0) {
-        return fail(ctx, "rc_resize: sort buffer allocation failed");
+    SortBufs &so = ctx->sort;
+    if (!so.hist.get()) {
+        CU_CHECK(ctx, so.hist.alloc(size_t(kMaxBounces) * kSortBins));
     }
+    if (!so.chunk_totals.get()) {
+        CU_CHECK(ctx, so.chunk_totals.alloc(size_t(kMaxBounces) * 64));
+    }
+    CU_CHECK(ctx, so.keys.alloc(n));
+    CU_CHECK(ctx, so.keys_sorted.alloc(n));
     ctx->ray_capacity = n;
     ctx->fb.w = w;
     ctx->fb.h = h;
@@ -1206,18 +1145,14 @@ int rc_upload_tables(rc_ctx *ctx, const uint32_t *pmj, int dims, int samples, co
     }
     cudaSetDevice(ctx->device);
     const size_t n = size_t(dims) * samples * 2;
-    if (dev_alloc(ctx, &ctx->d_pmj, n)) {
-        return 1;
-    }
-    CU_CHECK(ctx, cudaMemcpy(ctx->d_pmj, pmj, n * sizeof(uint32_t), cudaMemcpyHostToDevice));
+    CU_CHECK(ctx, ctx->d_pmj.alloc(n));
+    CU_CHECK(ctx, cudaMemcpy(ctx->d_pmj.get(), pmj, n * sizeof(uint32_t), cudaMemcpyHostToDevice));
     if (filter_table) {
         if (filter_table_size != kFilterTableSize) {
             return fail(ctx, "rc_upload_tables: filter table must have %d entries", kFilterTableSize);
         }
-        if (dev_alloc(ctx, &ctx->d_filter_table, size_t(kFilterTableSize))) {
-            return 1;
-        }
-        CU_CHECK(ctx, cudaMemcpy(ctx->d_filter_table, filter_table, kFilterTableSize * sizeof(float),
+        CU_CHECK(ctx, ctx->d_filter_table.alloc(kFilterTableSize));
+        CU_CHECK(ctx, cudaMemcpy(ctx->d_filter_table.get(), filter_table, kFilterTableSize * sizeof(float),
                                  cudaMemcpyHostToDevice));
     }
     ctx->have_tables = true;
@@ -1418,19 +1353,16 @@ namespace {
 // grow / shrink a node array to new_count records keeping the first `keep` ones (device-to-device)
 int resize_keep(rc_ctx *ctx, DevArray &a, uint32_t keep, uint32_t new_count) {
     const size_t want = size_t(new_count) * sizeof(WNode);
-    if (a.ptr && a.bytes == want) {
+    if (a.fits(want)) {
         return 0;
     }
-    void *fresh = nullptr;
-    CU_CHECK(ctx, cudaMalloc(&fresh, want ? want : 256));
-    if (a.ptr && keep != 0) {
-        CU_CHECK(ctx, cudaMemcpyAsync(fresh, a.ptr, size_t(keep) * sizeof(WNode), cudaMemcpyDeviceToDevice, ctx->stream));
+    DevArray fresh;
+    CU_CHECK(ctx, fresh.resize(want, new_count));
+    if (a.ptr() && keep != 0) {
+        CU_CHECK(ctx, cudaMemcpyAsync(fresh.ptr(), a.ptr(), size_t(keep) * sizeof(WNode), cudaMemcpyDeviceToDevice, ctx->stream));
     }
     CU_CHECK(ctx, cudaStreamSynchronize(ctx->stream));
-    cudaFree(a.ptr);
-    a.ptr = fresh;
-    a.bytes = want;
-    a.count = new_count;
+    a = std::move(fresh); // frees the old block
     return 0;
 }
 } // namespace
@@ -1442,15 +1374,15 @@ int rc_set_view_lut(rc_ctx *ctx, uint32_t view_transform, const uint32_t *lut, i
     }
     cudaSetDevice(ctx->device);
     CU_CHECK(ctx, cudaStreamSynchronize(ctx->stream));
-    if (ctx->last_xf.lut == ctx->d_view_lut[view_transform]) {
+    if (ctx->last_xf.lut == ctx->d_view_lut[view_transform].get()) {
         ctx->last_xf.lut = nullptr;
     }
-    cudaFree(ctx->d_view_lut[view_transform]);
-    ctx->d_view_lut[view_transform] = nullptr;
+    DevBuf<uint32_t> &table = ctx->d_view_lut[view_transform];
+    table.reset();
     if (lut) {
-        const size_t bytes = size_t(dims) * dims * dims * sizeof(uint32_t);
-        CU_CHECK(ctx, cudaMalloc(&ctx->d_view_lut[view_transform], bytes));
-        CU_CHECK(ctx, cudaMemcpy(ctx->d_view_lut[view_transform], lut, bytes, cudaMemcpyHostToDevice));
+        const size_t n = size_t(dims) * dims * dims;
+        CU_CHECK(ctx, table.alloc(n));
+        CU_CHECK(ctx, cudaMemcpy(table.get(), lut, n * sizeof(uint32_t), cudaMemcpyHostToDevice));
     }
     return 0;
 }
@@ -1543,7 +1475,7 @@ int rc_update_instances(rc_ctx *ctx, const rc_scene_view *sv, uint32_t first_nod
     }
     ctx->wnodes.count = ctx->dnodes.count = n_nodes;
     if (n_nodes > first_node) {
-        CU_CHECK(ctx, cudaMemcpyAsync(static_cast<WNode *>(ctx->wnodes.ptr) + first_node, nodes + first_node,
+        CU_CHECK(ctx, cudaMemcpyAsync(static_cast<WNode *>(ctx->wnodes.ptr()) + first_node, nodes + first_node,
                                       size_t(n_nodes - first_node) * sizeof(WNode), cudaMemcpyHostToDevice, ctx->stream));
         ctx->scene_h2d_bytes += size_t(n_nodes - first_node) * sizeof(WNode);
     }
@@ -1556,12 +1488,12 @@ int rc_update_instances(rc_ctx *ctx, const rc_scene_view *sv, uint32_t first_nod
     }
     if (n_nodes > first_node) {
         k_build_dnodes<<<((n_nodes - first_node) * 8 + 255) / 256, 256, 0, ctx->stream>>>(
-            static_cast<const WNode *>(ctx->wnodes.ptr), static_cast<WNode *>(ctx->dnodes.ptr), first_node, n_nodes);
+            static_cast<const WNode *>(ctx->wnodes.ptr()), static_cast<WNode *>(ctx->dnodes.ptr()), first_node, n_nodes);
     }
     if (n_inst != 0) {
         k_build_blas_roots<<<(n_inst + 255) / 256, 256, 0, ctx->stream>>>(
-            static_cast<const WNode *>(ctx->wnodes.ptr), static_cast<const MeshInstance *>(ctx->mesh_instances.ptr), n_inst,
-            n_nodes, static_cast<uint32_t *>(ctx->blas_roots.ptr));
+            static_cast<const WNode *>(ctx->wnodes.ptr()), static_cast<const MeshInstance *>(ctx->mesh_instances.ptr()), n_inst,
+            n_nodes, static_cast<uint32_t *>(ctx->blas_roots.ptr()));
     }
     CU_CHECK(ctx, cudaStreamSynchronize(ctx->stream)); // lts is a local
     CU_CHECK(ctx, cudaGetLastError());
@@ -1651,20 +1583,16 @@ void unet_tensor_shape(int i, int &channels, int &shift) {
 
 int unet_alloc_tensors(rc_ctx *ctx) {
     const int wr = (ctx->w + 15) / 16 * 16, hr = (ctx->h + 15) / 16 * 16;
-    if (ctx->unet_tw == wr && ctx->unet_th == hr && ctx->unet_t[0]) {
+    if (ctx->unet_tw == wr && ctx->unet_th == hr && ctx->unet_t[0].get()) {
         return 0;
-    }
-    for (float *&t : ctx->unet_t) {
-        cudaFree(t);
-        t = nullptr;
     }
     ctx->unet_tw = ctx->unet_th = 0;
     for (int i = 0; i < 15; ++i) {
         int c, sh;
         unet_tensor_shape(i, c, sh);
         const size_t n = size_t(wr >> sh) * size_t(hr >> sh) * size_t(c);
-        CU_CHECK(ctx, cudaMalloc(&ctx->unet_t[i], (n ? n : 1) * sizeof(float)));
-        CU_CHECK(ctx, cudaMemsetAsync(ctx->unet_t[i], 0, (n ? n : 1) * sizeof(float), ctx->stream));
+        CU_CHECK(ctx, ctx->unet_t[i].alloc(n ? n : 1));
+        CU_CHECK(ctx, cudaMemsetAsync(ctx->unet_t[i].get(), 0, (n ? n : 1) * sizeof(float), ctx->stream));
     }
     ctx->unet_tw = wr;
     ctx->unet_th = hr;
@@ -1692,20 +1620,13 @@ size_t unet_h_elems(int w, int h, int cs) { return size_t(w + 2) * size_t(h + 2)
 
 int unet_tc_alloc(rc_ctx *ctx) {
     const int wr = (ctx->w + 15) / 16 * 16, hr = (ctx->h + 15) / 16 * 16;
-    if (ctx->unet_htw == wr && ctx->unet_hth == hr && ctx->unet_hx0) {
+    if (ctx->unet_htw == wr && ctx->unet_hth == hr && ctx->unet_hx0.get()) {
         return 0;
     }
-    for (__half *&t : ctx->unet_ht) {
-        cudaFree(t);
-        t = nullptr;
-    }
-    cudaFree(ctx->unet_hx0);
-    cudaFree(ctx->unet_hs);
-    ctx->unet_hx0 = ctx->unet_hs = nullptr;
     ctx->unet_htw = ctx->unet_hth = 0;
-    auto alloc0 = [&](__half **p, size_t n) -> int {
-        CU_CHECK(ctx, cudaMalloc(p, n * sizeof(__half)));
-        CU_CHECK(ctx, cudaMemsetAsync(*p, 0, n * sizeof(__half), ctx->stream)); // borders and padded channels stay zero for good
+    auto alloc0 = [&](DevBuf<__half> &b, size_t n) -> int {
+        CU_CHECK(ctx, b.alloc(n));
+        CU_CHECK(ctx, cudaMemsetAsync(b.get(), 0, n * sizeof(__half), ctx->stream)); // borders and padded channels stay zero for good
         return 0;
     };
     for (int i = 0; i < 15; ++i) {
@@ -1714,12 +1635,12 @@ int unet_tc_alloc(rc_ctx *ctx) {
         if (unet_tc_writes_upsampled(i)) {
             --sh; // stored already up-sampled (the convolution's epilogue replicates)
         }
-        if (alloc0(&ctx->unet_ht[i], unet_h_elems(wr >> sh, hr >> sh, round_up_i(c, 64)))) {
+        if (alloc0(ctx->unet_ht[i], unet_h_elems(wr >> sh, hr >> sh, round_up_i(c, 64)))) {
             return 1;
         }
     }
     // network input (64-channel stride) and the pre-pooling output of the encoder convolutions (sized for level 0)
-    if (alloc0(&ctx->unet_hx0, unet_h_elems(wr, hr, 64)) || alloc0(&ctx->unet_hs, unet_h_elems(wr, hr, 128))) {
+    if (alloc0(ctx->unet_hx0, unet_h_elems(wr, hr, 64)) || alloc0(ctx->unet_hs, unet_h_elems(wr, hr, 128))) {
         return 1;
     }
     ctx->unet_htw = wr;
@@ -1763,11 +1684,11 @@ int unet_conv_tc(rc_ctx *ctx, int layer, const __half *in1, int cs1, const __hal
     CUtensorMap map_a1, map_a2, map_b;
     if (make_map(ctx, &map_a1, in1, cs1, rows, tc::kHaloRows) ||
         make_map(ctx, &map_a2, in2 ? in2 : in1, in2 ? cs2 : cs1, rows, tc::kHaloRows) ||
-        make_map(ctx, &map_b, ctx->unet_hw[layer], unet_tc_in_cs(layer), size_t(9) * n, n)) {
+        make_map(ctx, &map_b, ctx->unet_hw[layer].get(), unet_tc_in_cs(layer), size_t(9) * n, n)) {
         return 1;
     }
     tc::ConvTcParams p{};
-    p.bias = ctx->unet_hb[layer];
+    p.bias = ctx->unet_hb[layer].get();
     p.out = out;
     p.fb = ctx->fb;
     p.w = w;
@@ -1803,11 +1724,6 @@ int unet_conv_tc(rc_ctx *ctx, int layer, const __half *in1, int cs1, const __hal
         p.a_slots = 3;
         p.stages = std::min(tc::kMaxStages, (tc::kSmemBudget - p.a_slots * tc::kASlotBytes) / b_slot_bytes);
     }
-    static bool attr_set = false;
-    if (!attr_set) {
-        cudaFuncSetAttribute(tc::k_unet_conv_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        attr_set = true;
-    }
     const int grid = std::min(p.tiles, 2 * ctx->num_sms);
     tc::k_unet_conv_tc<<<grid, tc::kThreads, smem, ctx->stream>>>(map_a1, map_a2, map_b, p);
     return 0;
@@ -1826,16 +1742,16 @@ int unet_run_tc(rc_ctx *ctx, int pass, const rc_rect &r) {
         const __half *in1, *in2 = nullptr;
         int cs1, cs2 = 0;
         if (i == 0) {
-            tc::k_unet_feat_h<<<dim3((wr + 127) / 128, hr), 128, 0, s>>>(ctx->fb, ctx->unet_hx0, wr, hr, 64);
-            in1 = ctx->unet_hx0;
+            tc::k_unet_feat_h<<<dim3((wr + 127) / 128, hr), 128, 0, s>>>(ctx->fb, ctx->unet_hx0.get(), wr, hr, 64);
+            in1 = ctx->unet_hx0.get();
             cs1 = 64;
         } else {
             // decoder (L.up): the previous layer already stored its output up-sampled; the skip tensor (or the network
             // input) is the second K range of the same GEMM -- no gather pass
-            in1 = ctx->unet_ht[i - 1];
+            in1 = ctx->unet_ht[i - 1].get();
             cs1 = round_up_i(L.cin1, 64);
             if (L.up) {
-                in2 = skip_of[i] == -2 ? ctx->unet_hx0 : ctx->unet_ht[skip_of[i]];
+                in2 = skip_of[i] == -2 ? ctx->unet_hx0.get() : ctx->unet_ht[skip_of[i]].get();
                 cs2 = skip_of[i] == -2 ? 64 : round_up_i(L.cin2, 64);
             }
         }
@@ -1845,13 +1761,13 @@ int unet_run_tc(rc_ctx *ctx, int pass, const rc_rect &r) {
                 return 1;
             }
         } else if (L.pool) {
-            if (unet_conv_tc(ctx, i, in1, cs1, in2, cs2, w, h, ctx->unet_hs, out_cs, false, r)) {
+            if (unet_conv_tc(ctx, i, in1, cs1, in2, cs2, w, h, ctx->unet_hs.get(), out_cs, false, r)) {
                 return 1;
             }
             const int c8 = round_up_i(L.cout, 8) / 8;
             const size_t work = size_t(w >> 1) * size_t(h >> 1) * size_t(c8);
-            tc::k_unet_pool_h<<<unsigned((work + 255) / 256), 256, 0, s>>>(ctx->unet_hs, out_cs, ctx->unet_ht[i], out_cs, c8, w, h);
-        } else if (unet_conv_tc(ctx, i, in1, cs1, in2, cs2, w, h, ctx->unet_ht[i], out_cs, unet_tc_writes_upsampled(i), r)) {
+            tc::k_unet_pool_h<<<unsigned((work + 255) / 256), 256, 0, s>>>(ctx->unet_hs.get(), out_cs, ctx->unet_ht[i].get(), out_cs, c8, w, h);
+        } else if (unet_conv_tc(ctx, i, in1, cs1, in2, cs2, w, h, ctx->unet_ht[i].get(), out_cs, unet_tc_writes_upsampled(i), r)) {
             return 1;
         }
     }
@@ -1882,13 +1798,10 @@ int rc_unet_set_weights(rc_ctx *ctx, const rc_unet_layer layers[16]) {
                 }
             }
         }
-        cudaFree(ctx->unet_w[i]);
-        cudaFree(ctx->unet_b[i]);
-        ctx->unet_w[i] = ctx->unet_b[i] = nullptr;
-        CU_CHECK(ctx, cudaMalloc(&ctx->unet_w[i], w.size() * sizeof(float)));
-        CU_CHECK(ctx, cudaMalloc(&ctx->unet_b[i], b.size() * sizeof(float)));
-        CU_CHECK(ctx, cudaMemcpy(ctx->unet_w[i], w.data(), w.size() * sizeof(float), cudaMemcpyHostToDevice));
-        CU_CHECK(ctx, cudaMemcpy(ctx->unet_b[i], b.data(), b.size() * sizeof(float), cudaMemcpyHostToDevice));
+        CU_CHECK(ctx, ctx->unet_w[i].alloc(w.size()));
+        CU_CHECK(ctx, ctx->unet_b[i].alloc(b.size()));
+        CU_CHECK(ctx, cudaMemcpy(ctx->unet_w[i].get(), w.data(), w.size() * sizeof(float), cudaMemcpyHostToDevice));
+        CU_CHECK(ctx, cudaMemcpy(ctx->unet_b[i].get(), b.data(), b.size() * sizeof(float), cudaMemcpyHostToDevice));
         // tensor-core path: the fp16 bits as they came, [tap][cout padded to 16][input channel stride], zero padded
         const int n = round_up_i(L.cout, 16), in_cs = unet_tc_in_cs(i);
         std::vector<uint16_t> hw(size_t(9) * n * in_cs, 0);
@@ -1901,14 +1814,10 @@ int rc_unet_set_weights(rc_ctx *ctx, const rc_unet_layer layers[16]) {
                 }
             }
         }
-        cudaFree(ctx->unet_hw[i]);
-        cudaFree(ctx->unet_hb[i]);
-        ctx->unet_hw[i] = nullptr;
-        ctx->unet_hb[i] = nullptr;
-        CU_CHECK(ctx, cudaMalloc(&ctx->unet_hw[i], hw.size() * 2));
-        CU_CHECK(ctx, cudaMalloc(&ctx->unet_hb[i], hb.size() * sizeof(float)));
-        CU_CHECK(ctx, cudaMemcpy(ctx->unet_hw[i], hw.data(), hw.size() * 2, cudaMemcpyHostToDevice));
-        CU_CHECK(ctx, cudaMemcpy(ctx->unet_hb[i], hb.data(), hb.size() * sizeof(float), cudaMemcpyHostToDevice));
+        CU_CHECK(ctx, ctx->unet_hw[i].alloc(hw.size()));
+        CU_CHECK(ctx, ctx->unet_hb[i].alloc(hb.size()));
+        CU_CHECK(ctx, cudaMemcpy(ctx->unet_hw[i].get(), hw.data(), hw.size() * 2, cudaMemcpyHostToDevice));
+        CU_CHECK(ctx, cudaMemcpy(ctx->unet_hb[i].get(), hb.data(), hb.size() * sizeof(float), cudaMemcpyHostToDevice));
     }
     ctx->unet_ready = true;
     return 0;
@@ -1972,11 +1881,11 @@ int rc_denoise_unet(rc_ctx *ctx, int pass, const rc_rect *rect, uint32_t flags) 
         p.feat_in2 = in2_of[i] == -2;
         p.last = (i == kUNetLayers - 1);
         p.xf = ctx->last_xf;
-        p.in1 = in1_of[i] >= 0 ? ctx->unet_t[in1_of[i]] : nullptr;
-        p.in2 = in2_of[i] >= 0 ? ctx->unet_t[in2_of[i]] : nullptr;
-        p.weights = ctx->unet_w[i];
-        p.bias = ctx->unet_b[i];
-        p.out = (i < 15) ? ctx->unet_t[i] : nullptr;
+        p.in1 = in1_of[i] >= 0 ? ctx->unet_t[in1_of[i]].get() : nullptr;
+        p.in2 = in2_of[i] >= 0 ? ctx->unet_t[in2_of[i]].get() : nullptr;
+        p.weights = ctx->unet_w[i].get();
+        p.bias = ctx->unet_b[i].get();
+        p.out = (i < 15) ? ctx->unet_t[i].get() : nullptr;
         // the region on this level's grid: passes < 15 round the frame rect up to 16 first (RendererCPU.h:797-801)
         int x0 = r.x, y0 = r.y, x1 = r.x + r.w, y1 = r.y + r.h;
         if (i < 15) {
@@ -2012,56 +1921,40 @@ int rc_build_lbvh(rc_ctx *ctx, const float *boxes, uint32_t n, rc_lbvh_node *nod
     static_assert(sizeof(rc_lbvh_node) == sizeof(LbvhNode), "layout");
     cudaSetDevice(ctx->device);
     cudaStream_t s = ctx->stream;
-    float *d_boxes = nullptr, *d_bounds = nullptr;
-    uint32_t *d_codes = nullptr, *d_codes2 = nullptr, *d_ids = nullptr, *d_ids2 = nullptr, *d_parent = nullptr, *d_visits = nullptr;
-    LbvhNode *d_nodes = nullptr;
-    void *d_temp = nullptr;
+    DevBuf<float> d_boxes, d_bounds;
+    DevBuf<uint32_t> d_codes, d_codes2, d_ids, d_ids2, d_parent, d_visits;
+    DevBuf<LbvhNode> d_nodes;
+    if (d_boxes.alloc(size_t(n) * 6) != cudaSuccess || d_bounds.alloc(6) != cudaSuccess || d_codes.alloc(n) != cudaSuccess ||
+        d_codes2.alloc(n) != cudaSuccess || d_ids.alloc(n) != cudaSuccess || d_ids2.alloc(n) != cudaSuccess ||
+        d_parent.alloc(size_t(2) * n - 1) != cudaSuccess || d_visits.alloc(n) != cudaSuccess ||
+        d_nodes.alloc(size_t(2) * n - 1) != cudaSuccess) {
+        return fail(ctx, "rc_build_lbvh: out of device memory");
+    }
+    cudaMemcpyAsync(d_boxes.get(), boxes, size_t(n) * 6 * sizeof(float), cudaMemcpyHostToDevice, s);
+    const int init[6] = {0x7fffffff, 0x7fffffff, 0x7fffffff, int(0x80000000), int(0x80000000), int(0x80000000)};
+    cudaMemcpyAsync(d_bounds.get(), init, sizeof(init), cudaMemcpyHostToDevice, s);
+    cudaMemsetAsync(d_visits.get(), 0, size_t(n) * 4, s);
+    const unsigned blocks = (n + 255) / 256;
+    k_lbvh_bounds<<<min(blocks, 1024u), 256, 0, s>>>(d_boxes.get(), n, d_bounds.get());
+    k_lbvh_codes<<<blocks, 256, 0, s>>>(d_boxes.get(), n, d_bounds.get(), d_codes.get(), d_ids.get());
     size_t temp_bytes = 0;
-    int rc = 1;
-    do {
-        if (cudaMalloc(&d_boxes, size_t(n) * 6 * sizeof(float)) != cudaSuccess || cudaMalloc(&d_bounds, 6 * sizeof(float)) != cudaSuccess ||
-            cudaMalloc(&d_codes, n * 4) != cudaSuccess || cudaMalloc(&d_codes2, n * 4) != cudaSuccess ||
-            cudaMalloc(&d_ids, n * 4) != cudaSuccess || cudaMalloc(&d_ids2, n * 4) != cudaSuccess ||
-            cudaMalloc(&d_parent, (size_t(2) * n - 1) * 4) != cudaSuccess || cudaMalloc(&d_visits, size_t(n) * 4) != cudaSuccess ||
-            cudaMalloc(&d_nodes, (size_t(2) * n - 1) * sizeof(LbvhNode)) != cudaSuccess) {
-            fail(ctx, "rc_build_lbvh: out of device memory");
-            break;
-        }
-        cudaMemcpyAsync(d_boxes, boxes, size_t(n) * 6 * sizeof(float), cudaMemcpyHostToDevice, s);
-        const int init[6] = {0x7fffffff, 0x7fffffff, 0x7fffffff, int(0x80000000), int(0x80000000), int(0x80000000)};
-        cudaMemcpyAsync(d_bounds, init, sizeof(init), cudaMemcpyHostToDevice, s);
-        cudaMemsetAsync(d_visits, 0, size_t(n) * 4, s);
-        const unsigned blocks = (n + 255) / 256;
-        k_lbvh_bounds<<<min(blocks, 1024u), 256, 0, s>>>(d_boxes, n, d_bounds);
-        k_lbvh_codes<<<blocks, 256, 0, s>>>(d_boxes, n, d_bounds, d_codes, d_ids);
-        cub::DeviceRadixSort::SortPairs(nullptr, temp_bytes, d_codes, d_codes2, d_ids, d_ids2, int(n), 0, 30, s);
-        if (cudaMalloc(&d_temp, temp_bytes ? temp_bytes : 16) != cudaSuccess) {
-            fail(ctx, "rc_build_lbvh: out of device memory");
-            break;
-        }
-        cub::DeviceRadixSort::SortPairs(d_temp, temp_bytes, d_codes, d_codes2, d_ids, d_ids2, int(n), 0, 30, s);
-        k_lbvh_hierarchy<<<blocks, 256, 0, s>>>(d_codes2, int(n), d_nodes, d_parent);
-        k_lbvh_fit<<<blocks, 256, 0, s>>>(d_boxes, d_ids2, int(n), d_nodes, d_parent, d_visits);
-        cudaMemcpyAsync(nodes_out, d_nodes, (size_t(2) * n - 1) * sizeof(LbvhNode), cudaMemcpyDeviceToHost, s);
-        cudaMemcpyAsync(order_out, d_ids2, size_t(n) * 4, cudaMemcpyDeviceToHost, s);
-        const cudaError_t e = cudaStreamSynchronize(s);
-        if (e != cudaSuccess || cudaGetLastError() != cudaSuccess) {
-            fail(ctx, "rc_build_lbvh: %s", cudaGetErrorString(e));
-            break;
-        }
-        rc = 0;
-    } while (false);
-    cudaFree(d_boxes);
-    cudaFree(d_bounds);
-    cudaFree(d_codes);
-    cudaFree(d_codes2);
-    cudaFree(d_ids);
-    cudaFree(d_ids2);
-    cudaFree(d_parent);
-    cudaFree(d_visits);
-    cudaFree(d_nodes);
-    cudaFree(d_temp);
-    return rc;
+    cub::DeviceRadixSort::SortPairs(nullptr, temp_bytes, d_codes.get(), d_codes2.get(), d_ids.get(), d_ids2.get(), int(n), 0,
+                                    30, s);
+    DevBuf<uint8_t> d_temp;
+    if (d_temp.alloc(temp_bytes ? temp_bytes : 16) != cudaSuccess) {
+        return fail(ctx, "rc_build_lbvh: out of device memory");
+    }
+    cub::DeviceRadixSort::SortPairs(d_temp.get(), temp_bytes, d_codes.get(), d_codes2.get(), d_ids.get(), d_ids2.get(),
+                                    int(n), 0, 30, s);
+    k_lbvh_hierarchy<<<blocks, 256, 0, s>>>(d_codes2.get(), int(n), d_nodes.get(), d_parent.get());
+    k_lbvh_fit<<<blocks, 256, 0, s>>>(d_boxes.get(), d_ids2.get(), int(n), d_nodes.get(), d_parent.get(), d_visits.get());
+    cudaMemcpyAsync(nodes_out, d_nodes.get(), (size_t(2) * n - 1) * sizeof(LbvhNode), cudaMemcpyDeviceToHost, s);
+    cudaMemcpyAsync(order_out, d_ids2.get(), size_t(n) * 4, cudaMemcpyDeviceToHost, s);
+    const cudaError_t e = cudaStreamSynchronize(s);
+    if (e != cudaSuccess || cudaGetLastError() != cudaSuccess) {
+        return fail(ctx, "rc_build_lbvh: %s", cudaGetErrorString(e));
+    }
+    return 0;
 }
 
 int rc_denoise_nlm(rc_ctx *ctx, const rc_rect *rect, int iteration) {
@@ -2078,16 +1971,12 @@ int rc_denoise_nlm(rc_ctx *ctx, const rc_rect *rect, int iteration) {
     p.rx = r.x, p.ry = r.y, p.rw = r.w, p.rh = r.h;
     p.ex = r.x - kNlmExt, p.ey = r.y - kNlmExt, p.ew = r.w + 2 * kNlmExt, p.eh = r.h + 2 * kNlmExt;
     const size_t plane = size_t(p.ew) * p.eh;
-    if (ctx->nlm_scratch_elems < 3 * plane) {
-        cudaFree(ctx->nlm_scratch);
-        ctx->nlm_scratch = nullptr;
-        ctx->nlm_scratch_elems = 0;
-        CU_CHECK(ctx, cudaMalloc(&ctx->nlm_scratch, 3 * plane * sizeof(float4)));
-        ctx->nlm_scratch_elems = 3 * plane;
+    if (ctx->nlm_scratch.count() < 3 * plane) {
+        CU_CHECK(ctx, ctx->nlm_scratch.alloc(3 * plane));
     }
-    p.temp_final = ctx->nlm_scratch;
-    p.var_h = ctx->nlm_scratch + plane;
-    p.var_f = ctx->nlm_scratch + 2 * plane;
+    p.temp_final = ctx->nlm_scratch.get();
+    p.var_h = ctx->nlm_scratch.get() + plane;
+    p.var_f = ctx->nlm_scratch.get() + 2 * plane;
     p.variance_threshold = ctx->last_variance_threshold;
     p.iteration = iteration;
     p.xf = ctx->last_xf;
@@ -2450,7 +2339,7 @@ int rc_get_counters(rc_ctx *ctx, rc_counters *out) {
     cudaSetDevice(ctx->device);
     rc_sync(ctx);
     unsigned long long t[TOT_COUNT];
-    CU_CHECK(ctx, cudaMemcpy(t, ctx->d_totals, sizeof(t), cudaMemcpyDeviceToHost));
+    CU_CHECK(ctx, cudaMemcpy(t, ctx->d_totals.get(), sizeof(t), cudaMemcpyDeviceToHost));
     out->primary_rays = t[TOT_PRIMARY];
     out->secondary_rays = t[TOT_SECONDARY];
     out->shadow_rays = t[TOT_SHADOW];
@@ -2469,7 +2358,7 @@ int rc_reset_stats(rc_ctx *ctx) {
     memset(ctx->stats_us, 0, sizeof(ctx->stats_us));
     memset(ctx->kernel_ms, 0, sizeof(ctx->kernel_ms));
     memset(ctx->kernel_launches, 0, sizeof(ctx->kernel_launches));
-    CU_CHECK(ctx, cudaMemset(ctx->d_totals, 0, TOT_COUNT * sizeof(unsigned long long)));
+    CU_CHECK(ctx, cudaMemset(ctx->d_totals.get(), 0, TOT_COUNT * sizeof(unsigned long long)));
     return 0;
 }
 
@@ -2500,7 +2389,7 @@ int rc_stage_generate_primary_rays(rc_ctx *ctx, const rc_pass_desc *pass, void *
     if (fill_params(ctx, pass, p)) {
         return 1;
     }
-    CU_CHECK(ctx, cudaMemsetAsync(ctx->d_counters, 0, CNT_TOTAL * sizeof(uint32_t), ctx->stream));
+    CU_CHECK(ctx, cudaMemsetAsync(ctx->d_counters.get(), 0, CNT_TOTAL * sizeof(uint32_t), ctx->stream));
     const int n_pix_tiles = ((p.rect_w + 7) / 8) * ((p.rect_h + 3) / 4);
     k_raygen<<<(n_pix_tiles * 32 + 255) / 256, 256, 0, ctx->stream>>>(p, ctx->rays[0], ctx->hits);
     CU_CHECK(ctx, cudaStreamSynchronize(ctx->stream));
@@ -2530,7 +2419,7 @@ int rc_stage_generate_geo_rays(rc_ctx *ctx, const rc_pass_desc *pass, void *rays
     if (fill_params(ctx, pass, p) || ensure_geo_lists(ctx, pass)) {
         return 1;
     }
-    CU_CHECK(ctx, cudaMemsetAsync(ctx->d_counters, 0, CNT_TOTAL * sizeof(uint32_t), ctx->stream));
+    CU_CHECK(ctx, cudaMemsetAsync(ctx->d_counters.get(), 0, CNT_TOTAL * sizeof(uint32_t), ctx->stream));
     const int n_pix_tiles = ((p.rect_w + 7) / 8) * ((p.rect_h + 3) / 4);
     k_raygen_geo<<<(n_pix_tiles * 32 + 255) / 256, 256, 0, ctx->stream>>>(p, geo_params(ctx, pass), ctx->rays[0], ctx->hits);
     CU_CHECK(ctx, cudaStreamSynchronize(ctx->stream));
@@ -2564,7 +2453,7 @@ int rc_stage_trace_rays(rc_ctx *ctx, const rc_pass_desc *pass, void *rays, void 
     if (count == 0) {
         return 0;
     }
-    CU_CHECK(ctx, cudaMemsetAsync(ctx->d_counters, 0, CNT_TOTAL * sizeof(uint32_t), ctx->stream));
+    CU_CHECK(ctx, cudaMemsetAsync(ctx->d_counters.get(), 0, CNT_TOTAL * sizeof(uint32_t), ctx->stream));
     CU_CHECK(ctx, cudaStreamSynchronize(ctx->stream));
     if (upload_rays_aos(ctx, ctx->rays[0], static_cast<const RayAoS *>(rays), count) ||
         upload_hits_aos(ctx, ctx->hits, static_cast<const HitAoS *>(hits), count) ||
@@ -2603,7 +2492,7 @@ int rc_stage_shade(rc_ctx *ctx, const rc_pass_desc *pass, int primary, int bounc
     if (count == 0) {
         return 0;
     }
-    CU_CHECK(ctx, cudaMemsetAsync(ctx->d_counters, 0, CNT_TOTAL * sizeof(uint32_t), ctx->stream));
+    CU_CHECK(ctx, cudaMemsetAsync(ctx->d_counters.get(), 0, CNT_TOTAL * sizeof(uint32_t), ctx->stream));
     CU_CHECK(ctx, cudaStreamSynchronize(ctx->stream));
     if (upload_rays_aos(ctx, ctx->rays[0], static_cast<const RayAoS *>(rays), count) ||
         upload_hits_aos(ctx, ctx->hits, static_cast<const HitAoS *>(hits), count) ||
@@ -2653,7 +2542,7 @@ int rc_stage_trace_shadow_rays(rc_ctx *ctx, const rc_pass_desc *pass, const void
     if (count == 0) {
         return 0;
     }
-    CU_CHECK(ctx, cudaMemsetAsync(ctx->d_counters, 0, CNT_TOTAL * sizeof(uint32_t), ctx->stream));
+    CU_CHECK(ctx, cudaMemsetAsync(ctx->d_counters.get(), 0, CNT_TOTAL * sizeof(uint32_t), ctx->stream));
     CU_CHECK(ctx, cudaStreamSynchronize(ctx->stream));
     if (upload_shadow_aos(ctx, ctx->shadow, static_cast<const ShadowRayAoS *>(shadow_rays), count) ||
         set_counter(ctx, CNT_SHADOW + 0, uint32_t(count))) {
@@ -2683,8 +2572,8 @@ int rc_stage_sort_rays(rc_ctx *ctx, void *rays, int count, uint32_t *hashes_out)
     }
     KParams p;
     memset(&p, 0, sizeof(p));
-    p.counters = ctx->d_counters;
-    CU_CHECK(ctx, cudaMemsetAsync(ctx->d_counters, 0, CNT_TOTAL * sizeof(uint32_t), ctx->stream));
+    p.counters = ctx->d_counters.get();
+    CU_CHECK(ctx, cudaMemsetAsync(ctx->d_counters.get(), 0, CNT_TOTAL * sizeof(uint32_t), ctx->stream));
     CU_CHECK(ctx, cudaStreamSynchronize(ctx->stream));
     if (upload_rays_aos(ctx, ctx->rays[0], static_cast<const RayAoS *>(rays), count) ||
         set_counter(ctx, CNT_RAYS + 1, uint32_t(count))) {
@@ -2698,7 +2587,7 @@ int rc_stage_sort_rays(rc_ctx *ctx, void *rays, int count, uint32_t *hashes_out)
         return 1;
     }
     if (hashes_out) {
-        CU_CHECK(ctx, cudaMemcpy(hashes_out, ctx->sort.keys_sorted, size_t(count) * sizeof(uint32_t),
+        CU_CHECK(ctx, cudaMemcpy(hashes_out, ctx->sort.keys_sorted.get(), size_t(count) * sizeof(uint32_t),
                                  cudaMemcpyDeviceToHost));
     }
     return 0;

@@ -12,46 +12,20 @@
 // ~= 184 B/ray of HBM traffic, no multi-pass key shuffling.  Order inside a bin is arbitrary (and irrelevant).
 #pragma once
 
+#include "dev_buf.h"
 #include "rt_kernels.cuh"
 
 namespace rt {
 
+// Allocated by rc_resize: keys / keys_sorted per ray of the frame, hist / chunk_totals once.
 struct SortBufs {
-    uint32_t *keys = nullptr;        // key per input ray
-    uint32_t *keys_sorted = nullptr; // key per output ray (diagnostics / stage API)
-    uint32_t *hist = nullptr;        // kMaxBounces x kSortBins: one histogram per ray list, zeroed once per sample
-    uint32_t *chunk_totals = nullptr; // kMaxBounces x kSortChunks (k_sort_scan -> k_sort_scatter)
+    DevBuf<uint32_t> keys;         // key per input ray
+    DevBuf<uint32_t> keys_sorted;  // key per output ray (diagnostics / stage API)
+    DevBuf<uint32_t> hist;         // kMaxBounces x kSortBins: one histogram per ray list, zeroed once per sample
+    DevBuf<uint32_t> chunk_totals; // kMaxBounces x kSortChunks (k_sort_scan -> k_sort_scatter)
     float root_min[3] = {0, 0, 0};
     float inv_cell[3] = {1, 1, 1};
 };
-
-inline int alloc_sort_bufs(SortBufs &s, size_t n) {
-    cudaFree(s.keys);
-    cudaFree(s.keys_sorted);
-    s.keys = s.keys_sorted = nullptr;
-    if (!s.hist && cudaMalloc(&s.hist, size_t(kMaxBounces) * kSortBins * sizeof(uint32_t)) != cudaSuccess) {
-        return 1;
-    }
-    if (!s.chunk_totals && cudaMalloc(&s.chunk_totals, size_t(kMaxBounces) * 64 * sizeof(uint32_t)) != cudaSuccess) {
-        return 1;
-    }
-    if (n == 0) {
-        return 0;
-    }
-    if (cudaMalloc(&s.keys, n * sizeof(uint32_t)) != cudaSuccess ||
-        cudaMalloc(&s.keys_sorted, n * sizeof(uint32_t)) != cudaSuccess) {
-        return 1;
-    }
-    return 0;
-}
-
-inline void free_sort_bufs(SortBufs &s) {
-    cudaFree(s.keys);
-    cudaFree(s.keys_sorted);
-    cudaFree(s.hist);
-    cudaFree(s.chunk_totals);
-    s = SortBufs{};
-}
 
 inline void set_sort_bounds(SortBufs &s, const float bmin[3], const float bmax[3]) {
     for (int i = 0; i < 3; ++i) {
@@ -158,16 +132,16 @@ __global__ void __launch_bounds__(256) k_sort_scatter(const uint32_t *counters, 
 // KParams::sort_hist), so the 32 B/ray key pass is skipped; otherwise (stage API) they are built here.
 inline void sort_rays(SortBufs &s, const KParams &p, const RayBuf &src, const RayBuf &dst, int bounce, int num_sms,
                       bool have_hist, bool want_sorted_keys, cudaStream_t stream) {
-    uint32_t *hist = s.hist + size_t(bounce) * kSortBins;
+    uint32_t *hist = s.hist.get() + size_t(bounce) * kSortBins;
     if (!have_hist) {
         SortGrid g{s.root_min[0], s.root_min[1], s.root_min[2], s.inv_cell[0], s.inv_cell[1], s.inv_cell[2]};
         cudaMemsetAsync(hist, 0, kSortBins * sizeof(uint32_t), stream);
-        k_sort_hist<<<num_sms * 8, 256, 0, stream>>>(p.counters, bounce, src, g, s.keys, hist);
+        k_sort_hist<<<num_sms * 8, 256, 0, stream>>>(p.counters, bounce, src, g, s.keys.get(), hist);
     }
-    uint32_t *chunk_totals = s.chunk_totals + size_t(bounce) * kSortChunks;
+    uint32_t *chunk_totals = s.chunk_totals.get() + size_t(bounce) * kSortChunks;
     k_sort_scan<<<kSortChunks, 1024, 0, stream>>>(hist, chunk_totals);
-    k_sort_scatter<<<num_sms * 8, 256, 0, stream>>>(p.counters, bounce, src, dst, s.keys, hist, chunk_totals,
-                                                    want_sorted_keys ? s.keys_sorted : nullptr);
+    k_sort_scatter<<<num_sms * 8, 256, 0, stream>>>(p.counters, bounce, src, dst, s.keys.get(), hist, chunk_totals,
+                                                    want_sorted_keys ? s.keys_sorted.get() : nullptr);
 }
 
 } // namespace rt
