@@ -213,10 +213,14 @@ int rc_denoise_nlm(rc_ctx *ctx, const rc_rect *rect, int iteration);
  *   dec_conv4b, dec_conv3a, dec_conv3b, dec_conv2a, dec_conv2b, dec_conv1a, dec_conv1b, dec_conv0), each as fp16 OIHW
  *   weights [cout][cin][3][3] + fp16 biases [cout] -- the layout of OIDN's weight blobs the reference embeds
  *   (internal/precomputed/__oidn_weights_hdr_alb_nrm.inl).  Channel counts are checked against the network's shape.
- * rc_denoise_unet: pass 0..15 runs that pass over `rect` (frame coordinates; passes < 15 round it up to a multiple of
- *   16 like the reference), pass -1 runs all 16.  Pass 15 writes the filtered linear image to RC_BUF_RAW and its
- *   tonemapped version to RC_BUF_FINAL.  flags: RC_UNET_TENSOR_CORES (default path) computes the convolutions in fp16
- *   on the tensor cores with fp32 accumulation, RC_UNET_FP32 in fp32 FFMA (the parity anchor).  Blocking. */
+ * rc_denoise_unet: pass 0..15 runs that pass over `rect` (frame coordinates), pass -1 runs all 16.  Passes < 15
+ *   compute at least `rect` rounded outward to the 16-pixel grid of the frame (origin down, end up to a multiple of 16)
+ *   and may compute more of their tensor; pass 15 writes exactly the pixels of `rect`.  To filter a frame region by
+ *   region, call pass k for every region of a partition of the frame before pass k + 1 (pass-major): the regions of a
+ *   pass then write the whole intermediate tensor the next pass reads.  Pass 15 writes the filtered linear image to
+ *   RC_BUF_RAW and its tonemapped version to RC_BUF_FINAL.  flags: RC_UNET_TENSOR_CORES (default path) computes the
+ *   convolutions in fp16 on the tensor cores with fp32 accumulation, RC_UNET_FP32 in fp32 FFMA (the parity anchor).
+ *   Blocking. */
 typedef struct rc_unet_layer {
     const uint16_t *weights; /* fp16 bits, cout * cin * 9 */
     const uint16_t *bias;    /* fp16 bits, cout */
@@ -327,6 +331,18 @@ int rc_stage_trace_shadow_rays(rc_ctx *ctx, const rc_pass_desc *pass, const void
 int rc_stage_sort_rays(rc_ctx *ctx, void *rays, int count, uint32_t *hashes_out);
 /* overwrite the TEMP buffer (stage tests) */
 int rc_debug_fill_temp(rc_ctx *ctx, const float rgba[4]);
+/* overwrite frame plane `which` (RC_BUF_FINAL .. RC_BUF_TEMP; not an SH plane) with w*h RGBA floats from `src`, e.g. to
+ * feed the UNet synthetic colour / base-colour / depth-normals planes without rendering */
+int rc_debug_write_plane(rc_ctx *ctx, int which, const float *src);
+/* read back an intermediate tensor of the UNet path `flags` selects (RC_UNET_FP32 or RC_UNET_TENSOR_CORES), exactly as
+ * stored.  tensor 0..14: output of pass `tensor`; 15: the network input of the tensor-core path (9 features).
+ * dims = {rows, cols, channel stride} of the stored layout:
+ *   fp32 path:        (hr >> s, wr >> s, cout) with wr x hr the frame rounded up to 16 and s the tensor's down-scale
+ *   tensor-core path: (H + 2, W + 2, Cs) with the one-pixel zero border and the channel stride padded to 64; W x H is
+ *                     the stored grid, twice the level's grid for a tensor stored already up-sampled for the next pass
+ * Rows [row0, row0 + nrows) of that layout go to `dst` as floats (fp16 converted exactly); with dst == NULL only `dims`
+ * is filled.  Refused when the path has not run at the current rounded frame size, or tensor / rows are out of range. */
+int rc_debug_unet_tensor(rc_ctx *ctx, uint32_t flags, int tensor, int row0, int nrows, float *dst, int32_t dims[3]);
 /* sizeof() of the ABI structs as compiled into the library: 0 rc_array, 1 rc_scene_view, 2 rc_camera, 3 rc_rect,
  * 4 rc_pass_desc, 5 rc_counters; -1 for an unknown id.  Lets a binding verify its struct mirrors. */
 int rc_abi_sizeof(int which);

@@ -61,6 +61,8 @@ def load_library():
         "rc_stage_trace_shadow_rays": (C.c_int, [vp, P(capi.rc_pass_desc), vp, C.c_int, C.c_float]),
         "rc_stage_sort_rays": (C.c_int, [vp, vp, C.c_int, vp]),
         "rc_debug_fill_temp": (C.c_int, [vp, P(C.c_float)]),
+        "rc_debug_write_plane": (C.c_int, [vp, C.c_int, vp]),
+        "rc_debug_unet_tensor": (C.c_int, [vp, C.c_uint32, C.c_int, C.c_int, C.c_int, vp, P(C.c_int32)]),
         "rc_abi_sizeof": (C.c_int, [C.c_int]),
         "rc_host_alloc": (vp, [C.c_size_t]),
         "rc_host_free": (None, [vp]),
@@ -99,7 +101,7 @@ EXPORTED_SYMBOLS = [
     "rc_upload_tables", "rc_upload_scene", "rc_render", "rc_denoise_nlm", "rc_sync", "rc_readback", "rc_readback_required_samples",
     "rc_enable_stats", "rc_get_stats", "rc_get_counters", "rc_reset_stats", "rc_get_kernel_ms",
     "rc_stage_generate_primary_rays", "rc_stage_generate_geo_rays", "rc_stage_trace_rays", "rc_stage_shade", "rc_stage_trace_shadow_rays",
-    "rc_stage_sort_rays", "rc_debug_fill_temp", "rc_abi_sizeof", "rc_host_alloc", "rc_host_free", "rc_device_ptr",
+    "rc_stage_sort_rays", "rc_debug_fill_temp", "rc_debug_write_plane", "rc_debug_unet_tensor", "rc_abi_sizeof", "rc_host_alloc", "rc_host_free", "rc_device_ptr",
     "rc_event_record", "rc_event_elapsed_ms", "rc_readback_async", "rc_comm_init", "rc_comm_destroy", "rc_comm_last_error",
     "rc_comm_strip", "rc_comm_upload_scene", "rc_comm_upload_tables", "rc_comm_render", "rc_comm_sync", "rc_gather",
     "rc_gather_device", "rc_comm_get_counters", "rc_unet_set_weights", "rc_denoise_unet", "rc_build_lbvh", "rc_update_instances", "rc_scene_upload_bytes", "rc_set_view_lut",
@@ -314,3 +316,28 @@ class Context:
     def fill_temp(self, rgba=(0, 0, 0, 0)):
         arr = (C.c_float * 4)(*rgba)
         self._check(self.lib.rc_debug_fill_temp(self._ctx, arr), "rc_debug_fill_temp")
+
+    def debug_write_plane(self, which, array):
+        """Overwrite frame plane `which` (RC_BUF_FINAL .. RC_BUF_TEMP) with an (h, w, 4) float32 array."""
+        a = np.ascontiguousarray(array, dtype=np.float32)
+        if a.shape != (self.h, self.w, 4):
+            raise ValueError(f"debug_write_plane: expected shape {(self.h, self.w, 4)}, got {a.shape}")
+        self._check(self.lib.rc_debug_write_plane(self._ctx, which, _ptr(a)), "rc_debug_write_plane")
+
+    def debug_unet_dims(self, tensor, flags):
+        """(rows, cols, channel stride) of UNet tensor `tensor` of the path `flags` selects, as stored."""
+        dims = (C.c_int32 * 3)()
+        self._check(self.lib.rc_debug_unet_tensor(self._ctx, flags, tensor, 0, 0, None, dims), "rc_debug_unet_tensor")
+        return tuple(dims)
+
+    def debug_unet_tensor(self, tensor, flags, rows=None):
+        """UNet tensor `tensor` (0..14: output of that pass, 15: the tensor-core path's network input) of the path
+        `flags` selects, exactly as stored, as float32 (rows, cols, channel stride); rows = (row0, nrows) reads only
+        those rows of the stored layout."""
+        n, cols, cs = self.debug_unet_dims(tensor, flags)
+        row0, nrows = (0, n) if rows is None else (int(rows[0]), int(rows[1]))
+        out = np.empty((max(nrows, 0), cols, cs), dtype=np.float32)
+        dims = (C.c_int32 * 3)()
+        self._check(self.lib.rc_debug_unet_tensor(self._ctx, flags, tensor, row0, nrows, _ptr(out), dims),
+                    "rc_debug_unet_tensor")
+        return out
